@@ -23,6 +23,8 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# The benchmark may run from a read-only tree and leaves the tree as it found it: no bytecode caches written there.
+sys.dont_write_bytecode = True
 # One OpenMP thread per process (what torchrun sets for N > 1 anyway): the CPU legs run one forked worker per
 # core, and torch's intra-op pool inside each of them only oversubscribes the box (measured here: 116 k -> 180 k
 # env-steps/s for the reference path on 8 cores).  The GPU arm does no CPU compute.
@@ -337,6 +339,34 @@ def timed_generations(s, steps, flush, barrier, gen0=False, keep_prev_mu=None):
     return gen_ms, k1_ms, int(s.total_env_steps.item()) - before, wall
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, per_offspring, per_parameter):
+    """--dump-outputs: what the last timed generation handed its caller, as <out_dir>/<name>.npy (float32 arrays stay
+    float32, everything else becomes float64; integer ids below 2^53 are exact).  If the per-offspring arrays would take
+    the files past DUMP_LIMIT_BYTES, a fixed, seeded sample of offspring is written instead and its ids go to
+    offspring_ids.npy."""
+    import numpy as np
+
+    def host(t):
+        a = t.detach().cpu().numpy()
+        return a if a.dtype == np.float32 else a.astype(np.float64)
+    off = {k: host(t) for k, t in per_offspring.items()}
+    par = {k: host(t) for k, t in per_parameter.items()}
+    n = len(next(iter(off.values())))
+    room = DUMP_LIMIT_BYTES - sum(a.nbytes for a in par.values())
+    row = sum(a.itemsize for a in off.values())
+    if n * row > room:
+        keep = room // (row + 8)
+        ids = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        off = {k: a[ids] for k, a in off.items()}
+        off["offspring_ids"] = ids.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in dict(off, **par).items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def reduce_over_ranks(dev, world, gen_ms, k1_ms, n_steps):
     """max over ranks of the times, sum over ranks of the env steps (device-timed numbers, never wall clock)."""
     import torch
@@ -460,6 +490,9 @@ def run_b200(args):
     k1_rank_ms = {"max": k1_ms / args.steps, "mean": k1_mean_ms / args.steps}
     if s.exchange == "peer":
         eng.peer_check()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"fitness": s.fitness, "rank_order": s.order, "shaped_fitness": s.shaped},
+                     {"mu": s.parents[0], "adam_m": s.m, "adam_v": s.v})
 
     # ---------------- N > 1: every rank must hold the same bits, and a sample of the last generation must equal a 1-GPU rollout
     rank_consistency = None
@@ -487,7 +520,7 @@ def run_b200(args):
     # ---------------- the other regimes of the headline workload (SURVEY 8d: generation-0 and converged reported separately)
     regimes = {args.regime: regime_block(gen_ms, k1_ms, total_steps, args.steps, args.pop)}
     if not args.no_regimes:
-        k_other = max(3, min(args.steps, 20))
+        k_other = args.steps
         for reg in ("converged", "gen0", "from_scratch"):
             if reg in regimes:
                 continue
@@ -697,7 +730,8 @@ def measure_fp32_peak(device):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    ap.add_argument("--steps", type=int, default=100,
+                    help="timed generations of the headline workload (and of each of its other regimes)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--pop", type=int, default=P_DEFAULT)
@@ -711,7 +745,12 @@ def main():
                     help="N > 1: fitness exchange fused into K1 over NVLink peer memory (default) or an NCCL all-gather")
     ap.add_argument("--shard", default="cyclic", choices=["cyclic", "contiguous"],
                     help="N > 1: block-cyclic (default) or contiguous offspring-id ranges per rank")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed generations, write what the last one computed (fitness, rank order, shaped fitness, "
+                         "mu, Adam m and v) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     if args.impl == "reference":

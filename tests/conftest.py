@@ -13,15 +13,6 @@ GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "refonly: needs /root/reference (dev container only)")
-
-
-def pytest_collection_modifyitems(config, items):
-    have_ref = os.path.isdir("/root/reference/learning_strategies")
-    skip_ref = pytest.mark.skip(reason="/root/reference not present (GPU box)")
-    for item in items:
-        if "refonly" in item.keywords and not have_ref:
-            item.add_marker(skip_ref)
 
 
 @pytest.fixture(scope="session")

@@ -34,6 +34,29 @@ def test_reference_generation_port_from_state():
     assert steps == 2 * 500 and dt > 0
 
 
+def test_dump_outputs_writes_float_arrays_and_samples_above_the_cap(tmp_path, monkeypatch):
+    """--dump-outputs: float32 stays float32, every other dtype becomes float64; above the size cap the per-offspring arrays
+    are cut to the same seeded sample of offspring on every call, and their ids are written too."""
+    import torch
+    import bench
+    P, D = 5000, 226
+    off = {"fitness": torch.arange(P, dtype=torch.float64) * 0.5, "rank_order": torch.arange(P - 1, -1, -1, dtype=torch.int32)}
+    par = {"mu": torch.linspace(-1, 1, D, dtype=torch.float32)}
+    bench.dump_outputs(str(tmp_path / "full"), off, par)
+    got = {p.stem: np.load(p) for p in (tmp_path / "full").iterdir()}
+    assert sorted(got) == ["fitness", "mu", "rank_order"]
+    assert got["mu"].dtype == np.float32 and np.array_equal(got["mu"], par["mu"].numpy())
+    assert got["rank_order"].dtype == np.float64 and np.array_equal(got["rank_order"], np.arange(P - 1, -1, -1))
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", D * 4 + 1000 * 24)
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), off, par)
+    a = {p.stem: np.load(p) for p in (tmp_path / "a").iterdir()}
+    ids = a["offspring_ids"].astype(np.int64)
+    assert len(ids) == 1000 and np.all(np.diff(ids) > 0) and sum(x.nbytes for x in a.values()) <= bench.DUMP_LIMIT_BYTES
+    assert np.array_equal(a["fitness"], ids * 0.5) and np.array_equal(a["rank_order"], P - 1 - ids)
+    assert all(np.array_equal(a[k], np.load(tmp_path / "b" / (k + ".npy"))) for k in a)
+
+
 def test_reference_arm_line_keys():
     env = dict(os.environ, RANK="0")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0"],
