@@ -22,6 +22,10 @@ constexpr int SORT_WARPS = SORT_THREADS / 32;
 constexpr int SORT_ITEMS_SMALL = 4, SORT_ITEMS_LARGE = 16;
 __host__ __device__ constexpr int sort_tile(int items) { return SORT_THREADS * items; }
 
+// Every NaN, whatever its sign and payload, is keyed as +qNaN: above +inf, ties by descending index, as numpy ranks NaNs
+// (np.argsort puts them last).  The bit transform alone would send a NaN with the sign bit set to the bottom.
+constexpr unsigned long long SORT_KEY_NAN = 0x7ff8000000000000ull;
+
 // position p holds offspring i = n-1-p; key ascends when fitness descends
 __global__ void k_sort_init(const double *__restrict__ fitness, int n, int key_bits, double key_scale,
                             unsigned long long *__restrict__ keys, int *__restrict__ vals)
@@ -32,11 +36,12 @@ __global__ void k_sort_init(const double *__restrict__ fitness, int n, int key_b
     const double f = __dadd_rn(fitness[i], 0.0);   // -0.0 -> +0.0: numpy compares them equal
     unsigned long long k;
     if (key_bits == 0) {
-        const unsigned long long b = (unsigned long long)__double_as_longlong(f);
+        const unsigned long long b = isnan(f) ? SORT_KEY_NAN : (unsigned long long)__double_as_longlong(f);
         const unsigned long long asc = (b >> 63) ? ~b : (b | 0x8000000000000000ull);
         k = ~asc;
     } else {
-        // integer key in (-2^key_bits, 2^key_bits), biased to [1, 2^(key_bits+1))
+        // integer key in (-2^key_bits, 2^key_bits), biased to [1, 2^(key_bits+1)); never NaN: the host picks this path
+        // only for the step-count envs, whose fitness is a step total over E
         const long long v = __double2ll_rn(__dmul_rn(f, key_scale)) + (1ll << key_bits);
         k = ((2ull << key_bits) - 1ull) - (unsigned long long)v;
     }
@@ -165,10 +170,11 @@ __device__ __forceinline__ unsigned long long sort_key(const double *__restrict_
 {
     const double f = __dadd_rn(fitness[n - 1 - p], 0.0);   // position p holds offspring n-1-p; -0.0 -> +0.0
     if (key_bits == 0) {
-        const unsigned long long b = (unsigned long long)__double_as_longlong(f);
+        const unsigned long long b = isnan(f) ? SORT_KEY_NAN : (unsigned long long)__double_as_longlong(f);
         const unsigned long long asc = (b >> 63) ? ~b : (b | 0x8000000000000000ull);
         return ~asc;
     }
+    // integer keys: never NaN (step-count envs only, see k_sort_init)
     const long long v = __double2ll_rn(__dmul_rn(f, key_scale)) + (1ll << key_bits);
     return ((2ull << key_bits) - 1ull) - (unsigned long long)v;
 }

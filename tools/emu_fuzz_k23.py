@@ -1,7 +1,8 @@
 #!/usr/bin/env python
 """Differential fuzzing of K2 / K3 (host SIMT emulator, tests/simt_emu): ses_rank_desc in both builds (fused / separate
-kernels; float64 keys incl. +-inf, denormals, -0.0, constant vectors; integer keys) against np.flip(np.argsort(kind="stable")),
-and ses_update_openai / ses_materialize / ses_update_elite_mean with random layouts against the C twin.  No GPU needed.
+kernels; float64 keys incl. +-inf, denormals, -0.0, constant vectors, NaNs of both signs; integer keys) against
+np.flip(np.argsort(kind="stable")), and ses_update_openai / ses_materialize / ses_update_elite_mean with random layouts
+against the C twin.  No GPU needed.
 
     python tools/emu_fuzz_k23.py <first_case> <n_cases>      (4 600 cases, 0 mismatches at the end of round 1)
 """
@@ -21,13 +22,17 @@ for case in range(int(sys.argv[1]), int(sys.argv[1])+int(sys.argv[2])):
     rng=np.random.default_rng(case)
     os.environ["SES_K2_FUSED"]=str(case&1)
     n=int(rng.choice([2,3,31,32,33,255,256,257,1023,1024,1025, int(rng.integers(2,6000))]))
-    kind=rng.choice(["float","ties","int","const","inf"])
+    kind=rng.choice(["float","ties","int","const","inf","nan"])
     E=int(rng.choice([1,5,7])); ms=int(rng.choice([500,37,1]))
     eng=EmuEngine(population=n, group=n, eval_ep_num=E, max_step=ms, seed=case)
     if kind=="float": r=rng.normal(0,100,n)
     elif kind=="ties": r=np.round(rng.normal(0,2,n)); r[rng.random(n)<0.2]=-0.0
     elif kind=="const": r=np.full(n, float(rng.integers(-3,3)))
     elif kind=="inf": r=rng.normal(0,1,n); r[rng.random(n)<0.1]=np.inf; r[rng.random(n)<0.1]=-np.inf; r[rng.random(n)<0.05]=1e-310
+    elif kind=="nan":
+        r=rng.normal(0,1,n); r[rng.random(n)<0.1]=np.inf; r[rng.random(n)<0.1]=-np.inf
+        for b in (0x7ff8000000000000, 0xfff8000000000000, 0x7ff0000000000001, 0xfff0000000000123):
+            r[rng.random(n)<0.05]=np.array([b],np.uint64).view(np.float64)[0]
     else: r=rng.integers(E, E*ms+1, n)/E
     want=np.flip(np.argsort(r,kind="stable")).astype(np.int32)
     ok=np.array_equal(eng.rank_desc(r, full_key=True), want)
