@@ -96,7 +96,19 @@ int ses_rollout(ses_handle *h, uint32_t generation, float sigma, const float *pa
                 int64_t *steps_dev, double *trace_dev, int32_t *trace_actions_dev, int32_t n_trace,
                 void *stream);
 
-/* K2 -- replaces np.flip(np.argsort(rewards)) (offspring_strategies.py:112,234,380) with the tie
+/* Policy evaluation -- the GPU half of the reference's test.py (test.py:31-68; no rendering):
+ * n_pol policies x n_episodes episodes of this handle's env / network, common initial states.
+ *   policies_dev     [n_pol][D] f32, used as given (no noise, no antithetic pairing)
+ *   init_states_dev  optional [n_episodes][state_dim] f64 explicit initial states (verification mode);
+ *                    NULL -> episode m starts from Philox stream 2 at counter (m, 0, round, block), keyed
+ *                    by cfg.seed: every policy of the call sees the same episodes (DESIGN.md section 4.9)
+ *   returns_dev      [n_pol][n_episodes] f64: the episode's return (sequential sum of its step rewards)
+ *   lengths_dev      [n_pol][n_episodes] i32: its env steps (truncated at max_step as in training)
+ * Runs on this handle's device only; its strategy layout, shard and peers play no part. */
+int ses_evaluate(ses_handle *h, uint32_t round, const float *policies_dev, int32_t n_pol, int32_t n_episodes,
+                 const double *init_states_dev, double *returns_dev, int32_t *lengths_dev, void *stream);
+
+/* K2-- replaces np.flip(np.argsort(rewards)) (offspring_strategies.py:112,234,380) with the tie
  * order pinned to descending fitness, then DESCENDING index (== kind="stable"), and the centered
  * rank shaping (offspring_strategies.py:392-398).
  *   fitness_dev [n] f64 -> order_dev [n] i32 (order[0] = best); shaped_dev optional [n] f64.

@@ -119,7 +119,9 @@ __device__ __forceinline__ GruLaneConsts gru_lane_consts(const float4 *small, in
 //
 // One chunk of up to EC episodes (e0 .. e0 + ne - 1 of offspring `id`) stepped in lockstep by the calling warp; xh / obuf are
 // the warp's EC staging rows.  Returns the sum of the episode lengths (on every lane).
-template <int EC, bool SPEC, bool TRACE, int WREG = 0, class Smem>
+// EVAL (ses_evaluate): `id` is the virtual offspring (policy * layout.group + chunk), e0 the chunk's first episode of the policy;
+// initial states from STREAM_EVAL, and every episode stores its return and length.
+template <int EC, bool SPEC, bool TRACE, int WREG = 0, bool EVAL = false, class Smem>
 __device__ __forceinline__ int gru_run_chunk(Smem &sm, float2 (*xh)[HID], float (*obuf)[HID + 4], const GruLaneConsts &c,
                                              const RolloutParams &p, int id, int local_idx, int e0, int ne, int lane)
 {
@@ -137,7 +139,8 @@ __device__ __forceinline__ int gru_run_chunk(Smem &sm, float2 (*xh)[HID], float 
             const double *s0 = p.init_states + 4 * (e0 + ei);
             x = s0[0]; xd = s0[1]; th = s0[2]; thd = s0[3];
         } else {
-            cartpole_init(p.seed, p.init_mode, p.gen, (uint32_t)id, (uint32_t)(e0 + ei), x, xd, th, thd);
+            if constexpr (EVAL) cartpole_init(p.seed, 1, p.gen, 0u, (uint32_t)(e0 + ei), x, xd, th, thd, STREAM_EVAL);
+            else cartpole_init(p.seed, p.init_mode, p.gen, (uint32_t)id, (uint32_t)(e0 + ei), x, xd, th, thd);
         }
     }
     float h[EC];
@@ -293,13 +296,20 @@ __device__ __forceinline__ int gru_run_chunk(Smem &sm, float2 (*xh)[HID], float 
         alive_mask = __ballot_sync(FULL, alive);
     }
     // chunk total: lanes 0..ne-1 hold their episode lengths
+    if constexpr (EVAL) {
+        if (lane < ne) {
+            const size_t at = (size_t)(id / p.layout.group) * p.eval_episodes + e0 + lane;
+            p.eval_returns[at] = (double)nstep;
+            p.eval_lengths[at] = nstep;
+        }
+    }
     int n = lane < ne ? nstep : 0;
 #pragma unroll
     for (int o = 16; o; o >>= 1) n += __shfl_xor_sync(FULL, n, o);
     return n;
 }
 
-template <int EC, int WARPS, bool TRACE, bool SPEC = false, int WREG = 0>
+template <int EC, int WARPS, bool TRACE, bool SPEC = false, int WREG = 0, bool EVAL = false>
 __global__ void __launch_bounds__(WARPS * 32, 2) k_rollout_cartpole_gru(const RolloutParams p)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -320,6 +330,12 @@ __global__ void __launch_bounds__(WARPS * 32, 2) k_rollout_cartpole_gru(const Ro
         gru_load_weights(sm, p, id, local_idx, lane, 32);
         __syncwarp();
         const GruLaneConsts c = gru_lane_consts(sm.small, lane);
+        if constexpr (EVAL) {                                      // one chunk of p.E == EC episodes, the policy's last one partial
+            const int e0 = (id % p.layout.group) * p.E;
+            warp_steps += (unsigned long long)gru_run_chunk<EC, SPEC, false, WREG, true>(sm, sm.xh, sm.obuf, c, p, id, local_idx, e0,
+                                                                                          min(p.E, p.eval_episodes - e0), lane);
+            continue;
+        }
         long long total_steps = 0;
         for (int e0 = 0; e0 < p.E; e0 += EC)
             total_steps += gru_run_chunk<EC, SPEC, TRACE, WREG>(sm, sm.xh, sm.obuf, c, p, id, local_idx, e0, min(EC, p.E - e0), lane);
@@ -424,25 +440,27 @@ static int launch_rollout_cartpole_gru_pair(int num_sms, int ctas_per_sm, const 
 }
 #endif  // SES_BUILD_TESTS
 
-template <int EC>
+template <int EC, bool EVAL = false>
 static int launch_rollout_cartpole_gru_ec(int num_sms, int ctas_per_sm, const RolloutParams &rp, bool trace, cudaStream_t st,
                                           int64_t *launches, char *err, size_t errlen)
 {
     constexpr int WARPS = 4;
     const size_t smem = WARPS * sizeof(GruWarpSmem<EC>);
+    void (*kern)(const RolloutParams);
     // the product's kernel: speculative physics (SPEC, -5 %) with the n-gate table in registers (WREG = 1, another -3.7 %:
     // 4.14 ms at P = 4097 converged); the test build keeps the others selectable: SES_GRU_VARIANT 0 plain, 1 SPEC with every
     // table in shared memory, 3 the default, 4 SPEC with W_hh's r/z table in registers as well (255 registers, slower)
 #ifdef SES_BUILD_TESTS
     const char *ev = getenv("SES_GRU_VARIANT");                       // read per launch: tests switch it inside one process
     const int spec = ev && *ev ? atoi(ev) : 3;
-    auto kern = spec == 1 ? (trace ? k_rollout_cartpole_gru<EC, WARPS, true, true> : k_rollout_cartpole_gru<EC, WARPS, false, true>)
+    kern = spec == 1 ? (trace ? k_rollout_cartpole_gru<EC, WARPS, true, true> : k_rollout_cartpole_gru<EC, WARPS, false, true>)
               : spec == 4 ? (trace ? k_rollout_cartpole_gru<EC, WARPS, true, true, 2> : k_rollout_cartpole_gru<EC, WARPS, false, true, 2>)
               : spec == 0 ? (trace ? k_rollout_cartpole_gru<EC, WARPS, true, false> : k_rollout_cartpole_gru<EC, WARPS, false, false>)
                           : (trace ? k_rollout_cartpole_gru<EC, WARPS, true, true, 1> : k_rollout_cartpole_gru<EC, WARPS, false, true, 1>);
 #else
-    auto kern = trace ? k_rollout_cartpole_gru<EC, WARPS, true, true, 1> : k_rollout_cartpole_gru<EC, WARPS, false, true, 1>;
+    kern = trace ? k_rollout_cartpole_gru<EC, WARPS, true, true, 1> : k_rollout_cartpole_gru<EC, WARPS, false, true, 1>;
 #endif
+    if constexpr (EVAL) kern = k_rollout_cartpole_gru<EC, WARPS, false, true, 1, true>;      // the product's kernel, evaluation instance
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     int per_sm = 0;
     if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, WARPS * 32, smem);

@@ -126,12 +126,13 @@ struct MountainCarEnv {
     static constexpr bool LANES32_OK = false;     // the launcher may give all 32 lanes episodes (rollout_slots.cuh scheduler)
     struct State { double pos, vel, ret; };
 
+    template <uint32_t STREAM = STREAM_INIT>
     __device__ static __forceinline__ void init(State &s, const RolloutParams &p, int id, int ep)
     {
         if (p.init_states) {
             s.pos = p.init_states[2 * ep]; s.vel = p.init_states[2 * ep + 1];
         } else {
-            const uint4 r = philox4x32_10((uint32_t)ep, p.init_mode ? (uint32_t)id : 0u, p.init_mode ? p.gen : 0u, 0u, p.seed, STREAM_INIT);
+            const uint4 r = philox4x32_10((uint32_t)ep, p.init_mode ? (uint32_t)id : 0u, p.init_mode ? p.gen : 0u, 0u, p.seed, STREAM);
             s.pos = __dsub_rn(__dmul_rn(unit64(r.x), 0.2), 0.6);       // U(-0.6, -0.4)
             s.vel = 0.0;
         }
@@ -186,12 +187,13 @@ struct PendulumEnv {
     static constexpr double PI = 3.141592653589793;
     struct State { double th, thd, ret; };
 
+    template <uint32_t STREAM = STREAM_INIT>
     __device__ static __forceinline__ void init(State &s, const RolloutParams &p, int id, int ep)
     {
         if (p.init_states) {
             s.th = p.init_states[2 * ep]; s.thd = p.init_states[2 * ep + 1];
         } else {                                                       // uniform(-[pi, 1], [pi, 1])
-            const uint4 r = philox4x32_10((uint32_t)ep, p.init_mode ? (uint32_t)id : 0u, p.init_mode ? p.gen : 0u, 0u, p.seed, STREAM_INIT);
+            const uint4 r = philox4x32_10((uint32_t)ep, p.init_mode ? (uint32_t)id : 0u, p.init_mode ? p.gen : 0u, 0u, p.seed, STREAM);
             s.th = __dsub_rn(__dmul_rn(unit64(r.x), __dmul_rn(2.0, PI)), PI);
             s.thd = __dsub_rn(__dmul_rn(unit64(r.y), 2.0), 1.0);
         }
@@ -259,13 +261,14 @@ struct AcrobotEnv {
     // by the next step's observation and first RK4 stage (same function, same argument: same bits as recomputing)
     struct State { double s[4]; double sc[4]; double ret; };
 
+    template <uint32_t STREAM = STREAM_INIT>
     __device__ static __forceinline__ void init(State &st, const RolloutParams &p, int id, int ep)
     {
         if (p.init_states) {
 #pragma unroll
             for (int k = 0; k < 4; ++k) st.s[k] = p.init_states[4 * ep + k];
         } else {
-            const uint4 r = philox4x32_10((uint32_t)ep, p.init_mode ? (uint32_t)id : 0u, p.init_mode ? p.gen : 0u, 0u, p.seed, STREAM_INIT);
+            const uint4 r = philox4x32_10((uint32_t)ep, p.init_mode ? (uint32_t)id : 0u, p.init_mode ? p.gen : 0u, 0u, p.seed, STREAM);
             st.s[0] = __dsub_rn(__dmul_rn(unit64(r.x), 0.2), 0.1);       // U(-0.1, 0.1)^4
             st.s[1] = __dsub_rn(__dmul_rn(unit64(r.y), 0.2), 0.1);
             st.s[2] = __dsub_rn(__dmul_rn(unit64(r.z), 0.2), 0.1);

@@ -89,7 +89,9 @@ __device__ __forceinline__ float fc2_row_blocks(const float *w, const float *x, 
     return a;
 }
 
-template <class Env, int EC, int WARPS, bool TRACE>
+// EVAL (ses_evaluate): one chunk of p.E == EC episodes per virtual offspring (policy * layout.group + chunk), the policy's last
+// chunk partial; initial states from STREAM_EVAL, and every episode stores its return and length instead of a fitness.
+template <class Env, int EC, int WARPS, bool TRACE, bool EVAL = false>
 __global__ void __launch_bounds__(WARPS * 32) k_rollout_gru_generic(const RolloutParams p)
 {
     using Smem = GruGenSmem<Env, EC>;
@@ -128,10 +130,12 @@ __global__ void __launch_bounds__(WARPS * 32) k_rollout_gru_generic(const Rollou
 
         double total = 0.0;                                           // sum over episodes, in episode order, of the episode returns
         long long total_steps = 0;
+        [[maybe_unused]] const int m0 = EVAL ? (id % p.layout.group) * p.E : 0;     // EVAL: the chunk's first episode
         for (int e0 = 0; e0 < p.E; e0 += EC) {
-            const int ne = min(EC, p.E - e0);
+            const int ne = EVAL ? min(EC, p.eval_episodes - m0) : min(EC, p.E - e0);
             typename Env::State st;                                    // lane e < ne: episode e0 + e (other lanes: a harmless copy)
-            Env::init(st, p, id, e0 + (lane < ne ? lane : 0));
+            if constexpr (EVAL) Env::template init<STREAM_EVAL>(st, p, 0, m0 + (lane < ne ? lane : 0));
+            else Env::init(st, p, id, e0 + (lane < ne ? lane : 0));
             bool alive = lane < ne;
             int nstep = 0;
             float h[V];
@@ -233,6 +237,13 @@ __global__ void __launch_bounds__(WARPS * 32) k_rollout_gru_generic(const Rollou
                 }
                 alive_mask = __ballot_sync(FULL, alive);
             }
+            if constexpr (EVAL) {
+                if (lane < ne) {
+                    const size_t at = (size_t)(id / p.layout.group) * p.eval_episodes + m0 + lane;
+                    p.eval_returns[at] = st.ret;
+                    p.eval_lengths[at] = nstep;
+                }
+            }
             // returns of the chunk's episodes in episode order; steps
 #pragma unroll
             for (int e = 0; e < EC; ++e) {
@@ -245,7 +256,7 @@ __global__ void __launch_bounds__(WARPS * 32) k_rollout_gru_generic(const Rollou
             total_steps += n;
         }
         warp_steps += (unsigned long long)total_steps;
-        if (lane == 0) {
+        if (lane == 0 && !EVAL) {
             p.steps[id] = total_steps;
             publish_fitness(p, id, __ddiv_rn(total, (double)p.E));
         }
@@ -261,13 +272,14 @@ struct GruGenConfig {
     static constexpr int WARPS = 3;
 };
 
-template <class Env>
+template <class Env, bool EVAL = false>
 static int launch_rollout_gru_generic(int num_sms, int ctas_per_sm, const RolloutParams &rp, bool trace, cudaStream_t st, int64_t *launches,
                                       char *err, size_t errlen)
 {
     constexpr int EC = GruGenConfig<Env>::EC, WARPS = GruGenConfig<Env>::WARPS;
     const size_t smem = WARPS * sizeof(GruGenSmem<Env, EC>);
-    auto kern = trace ? k_rollout_gru_generic<Env, EC, WARPS, true> : k_rollout_gru_generic<Env, EC, WARPS, false>;
+    auto kern = EVAL ? k_rollout_gru_generic<Env, EC, WARPS, false, true>
+              : trace ? k_rollout_gru_generic<Env, EC, WARPS, true> : k_rollout_gru_generic<Env, EC, WARPS, false>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     int per_sm = 0;
     if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, WARPS * 32, smem);

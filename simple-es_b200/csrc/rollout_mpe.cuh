@@ -94,6 +94,7 @@ struct SpreadEnv {
         double ret;                                          // sequential sum of the episode's team rewards
     };
 
+    template <uint32_t STREAM = STREAM_INIT>
     __device__ static __forceinline__ void init(State &s, const RolloutParams &p, int id, int ep)
     {
         double v[4 * N];
@@ -104,7 +105,7 @@ struct SpreadEnv {
 #pragma unroll
             for (int b = 0; b < N; ++b) {
                 const uint4 r = philox4x32_10((uint32_t)ep, p.init_mode ? (uint32_t)id : 0u, p.init_mode ? p.gen : 0u, (uint32_t)b,
-                                              p.seed, STREAM_INIT);
+                                              p.seed, STREAM);
                 const double k32 = 2.3283064365386963e-10;
                 v[4 * b + 0] = __dsub_rn(__dmul_rn(__dmul_rn(__dadd_rn((double)r.x, 0.5), k32), 2.0), 1.0);
                 v[4 * b + 1] = __dsub_rn(__dmul_rn(__dmul_rn(__dadd_rn((double)r.y, 0.5), k32), 2.0), 1.0);

@@ -25,7 +25,7 @@
 //
 // An Env type provides:
 //   D, NQ, STATE_DIM, N_AGENTS, UNIT_REWARD (reward == 1.0 per step: fitness = steps / E exactly)
-//   struct State;  init(State&, p, id, ep);
+//   struct State;  init<STREAM = STREAM_INIT>(State&, p, id, ep)
 //   store_quad<S>(w[NQ][S], q, s, float4)   place flat parameter quad q of slot s (an Env may permute the table)
 //   bind<S>(State&, w[NQ][S], slot)          a lane was handed an episode of `slot` (an Env may cache weights in registers)
 //   step<S>(State&, w[NQ][S], slot, p, int *actions) -> done   (also adds the step reward to State::ret)
@@ -89,6 +89,11 @@ struct RolloutParams {
     int tail_start;              // episodes [0, tail_start) are handed out in whole offspring (queue A = work_counter[0]), the rest --
                                  // EPISODE_UNITS envs: the last round's worth -- in exact numbers (queue B = work_counter[WORK_COUNTER_TAIL])
     PeerSync sync;               // sync.world > 1: the launch ends with the peer flag barrier (slot kernels)
+    // policy evaluation (the EVAL instances, ses_evaluate): offspring id = policy * layout.group + chunk, a chunk is episodes
+    // [chunk E, chunk E + E) of the policy, clipped to eval_episodes
+    double *eval_returns;        // [n_pol][eval_episodes] return of every episode
+    int *eval_lengths;           // [n_pol][eval_episodes] its env steps
+    int eval_episodes;
 };
 
 constexpr int MAX_E = 32;
@@ -142,12 +147,17 @@ template <class Env> struct EnvEpisodeUnits<Env, decltype((void)Env::EPISODE_UNI
 // is emitted directly.  EPISODE_UNITS envs (reward 1 per step: the return is an integer step count) may have run parts of an
 // offspring in different warps: each part adds its steps, then its episode count, to the offspring's pair in ep_acc; the part
 // that completes the count emits the sum (integer addition: exact in any order) and clears the pair for the next launch.
-template <class Env, class Smem>
+// EVAL: every episode stored its return and length when it ended; nothing is left to emit.
+template <class Env, bool EVAL = false, class Smem>
 __device__ __forceinline__ void retire_slot(Smem &sm, const RolloutParams &p, int s, unsigned long long &warp_steps)
 {
     const int id = sm.off_id[s];
     const int stp = sm.steps[s];
     warp_steps += (unsigned long long)stp;
+    if constexpr (EVAL) {
+        sm.off_id[s] = -1;
+        return;
+    }
     bool whole = true;
     if constexpr (EnvEpisodeUnits<Env>::value) whole = sm.ep_cnt[s] == p.E;
     if (whole) {
@@ -241,7 +251,9 @@ __device__ __noinline__ void split_phase(Smem *smp, int pomdp, int max_step, int
 
 // PEER: the instance launched when the launch ends with the peer flag barrier (sentinel CTA + one atomic at the workers' end); a
 // separate instance so that single-GPU launches keep the exact code they have without it.
-template <class Env, int S, int WARPS, bool TRACE, bool PEER = false>
+// EVAL: the policy-evaluation instance (ses_evaluate): unperturbed policies, STREAM_EVAL initial states, per-episode returns and
+// lengths instead of fitness; no straggler phase.  Separate so that the training instances keep their code.
+template <class Env, int S, int WARPS, bool TRACE, bool PEER = false, bool EVAL = false>
 __global__ void __launch_bounds__(WARPS * 32) k_rollout_slots(const RolloutParams p)
 {
     using Smem = SlotSmem<Env, S, !Env::UNIT_REWARD>;
@@ -300,7 +312,7 @@ __global__ void __launch_bounds__(WARPS * 32) k_rollout_slots(const RolloutParam
             if (lane < S) {
                 my_id = sm.off_id[lane];
                 if (my_id >= 0 && sm.ep_done[lane] == sm.ep_cnt[lane]) {   // every episode of the slot has ended
-                    retire_slot<Env>(sm, p, lane, warp_steps);
+                    retire_slot<Env, EVAL>(sm, p, lane, warp_steps);
                     my_id = -1;
                 }
             }
@@ -374,7 +386,9 @@ __global__ void __launch_bounds__(WARPS * 32) k_rollout_slots(const RolloutParam
                 const bool fill = ((empty_mask >> lane) & 1u) && my_rank < n_off;
                 if (fill) {
                     const int ol = off0 + my_rank;
-                    const int lo = max(base, ol * p.E) - ol * p.E, hi = min(base + got, (ol + 1) * p.E) - ol * p.E;
+                    const int lo = max(base, ol * p.E) - ol * p.E;
+                    int hi = min(base + got, (ol + 1) * p.E) - ol * p.E;
+                    if constexpr (EVAL) hi = min(hi, p.eval_episodes - (ol % p.layout.group) * p.E);   // a partial last chunk
                     sm.off_id[lane] = p.shard.local_to_id(ol);
                     sm.ep_first[lane] = lo;
                     sm.ep_cnt[lane] = hi - lo;
@@ -426,7 +440,8 @@ __global__ void __launch_bounds__(WARPS * 32) k_rollout_slots(const RolloutParam
             __syncwarp();
             if (my_slot >= 0) {
                 slot = my_slot; ep = my_ep; nstep = 0;
-                Env::init(st, p, sm.off_id[my_slot], my_ep);
+                if constexpr (EVAL) Env::template init<STREAM_EVAL>(st, p, 0, (sm.off_id[my_slot] % p.layout.group) * p.E + my_ep);
+                else Env::init(st, p, sm.off_id[my_slot], my_ep);
                 Env::template bind<S>(st, sm.w, my_slot);
             }
             __syncwarp();
@@ -434,7 +449,7 @@ __global__ void __launch_bounds__(WARPS * 32) k_rollout_slots(const RolloutParam
             if (rerun) continue;                                   // queue A ran dry under this request: ask queue B for the rest
             const unsigned act_mask = __ballot_sync(FULL, slot >= 0);
             if (act_mask == 0) break;                              // queue empty and every lane idle
-            if constexpr (EnvSplit<Env>::value && !TRACE) {
+            if constexpr (EnvSplit<Env>::value && !TRACE && !EVAL) {
                 // nothing left to hand out (queue empty, every pending pair has a lane) and few episodes running: leave the
                 // throughput loop for the straggler phase below
                 if (p.split_ok && !more && acc <= n_idle && __popc(act_mask) <= 16) { to_split = true; break; }
@@ -457,7 +472,15 @@ __global__ void __launch_bounds__(WARPS * 32) k_rollout_slots(const RolloutParam
                 }
             }
             if (done) {
-                if constexpr (!Env::UNIT_REWARD) sm.ret[slot][ep] = st.ret;
+                if constexpr (EVAL) {
+                    const int vid = sm.off_id[slot];
+                    const size_t at = (size_t)(vid / p.layout.group) * p.eval_episodes + (vid % p.layout.group) * p.E + ep;
+                    if constexpr (Env::UNIT_REWARD) p.eval_returns[at] = (double)nstep;
+                    else p.eval_returns[at] = st.ret;
+                    p.eval_lengths[at] = nstep;
+                } else if constexpr (!Env::UNIT_REWARD) {
+                    sm.ret[slot][ep] = st.ret;
+                }
                 atomicAdd(&sm.steps[slot], nstep);
                 atomicAdd(&sm.ep_done[slot], 1);
                 slot = -1;
@@ -468,7 +491,7 @@ __global__ void __launch_bounds__(WARPS * 32) k_rollout_slots(const RolloutParam
         // to retire and refill); otherwise idle lanes stay idle and the warp keeps stepping
         sched = __ballot_sync(FULL, just_done) != 0;
     }
-    if constexpr (EnvSplit<Env>::value && !TRACE) {
+    if constexpr (EnvSplit<Env>::value && !TRACE && !EVAL) {
         // ------------------------------------------------------------------ straggler phase (kept out of the loop above so
         // that its code does not touch the throughput loop's register allocation and schedule)
         if (to_split) {

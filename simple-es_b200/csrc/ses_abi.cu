@@ -109,6 +109,7 @@ struct ses_handle {
     int spread_slots8 = 0;
     int k1_split = 1;
     int k1_sparse = 1;
+    int *eval_counter = nullptr;   // work counter of ses_evaluate's launches (allocated by the first call)
 
     int64_t launches = 0;
 };
@@ -241,6 +242,7 @@ extern "C" int ses_destroy(ses_handle *h)
     cudaFree(h->h_parents); cudaFree(h->h_m); cudaFree(h->h_v);
     cudaFree(h->h_fitness); cudaFree(h->h_shaped); cudaFree(h->h_steps); cudaFree(h->h_order); cudaFree(h->h_total);
     cudaFree(h->e_parents); cudaFree(h->e_out); cudaFree(h->e_fitness); cudaFree(h->e_steps); cudaFree(h->e_order); cudaFree(h->e_total);
+    cudaFree(h->eval_counter);
     delete h;
     return 0;
 }
@@ -458,6 +460,93 @@ extern "C" int ses_rollout(ses_handle *h, uint32_t generation, float sigma, cons
     }
     if (c.n_agents == 2) return launch_slots<SpreadEnv<2>, 8>(h, rp, need_warps, tr, st);
     return launch_slots<SpreadEnv<3>, 8>(h, rp, need_warps, tr, st);
+}
+
+// ------------------------------------------------------------------------------------------------
+// policy evaluation (DESIGN.md section 4.9): the EVAL instances of the K1 kernels
+// ------------------------------------------------------------------------------------------------
+// The slot kernel with chunks of E = 32 episodes: one chunk fills a warp.  Whole chunks only (queue A), so a chunk's clipped
+// episode count is exact; no sparse warps, no straggler phase.
+template <class Env, int SL, int WARPS = 4>
+static int launch_eval_slots(ses_handle *h, RolloutParams &rp, cudaStream_t st)
+{
+    using Smem = SlotSmem<Env, SL, !Env::UNIT_REWARD>;
+    auto kernel = k_rollout_slots<Env, SL, WARPS, false, false, true>;
+    const size_t smem = WARPS * sizeof(Smem);
+    CU(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int per_sm = 0;
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, WARPS * 32, smem));
+    if (per_sm < 1) return fail("evaluation kernel does not fit on an SM (smem %zu B)", smem);
+    rp.slots_cap = SL;
+    rp.lanes_used = 32;
+    rp.tail_start = rp.shard.n_local * rp.E;
+    const int need = (rp.shard.n_local + WARPS - 1) / WARPS;                  // one chunk per warp at most at a time
+    int grid = per_sm * h->num_sms;
+    if (grid > need) grid = need;
+    kernel<<<grid, WARPS * 32, smem, st>>>(rp);
+    CU(cudaGetLastError());
+    h->launches += 1;
+    return 0;
+}
+
+// episodes per chunk (virtual offspring) of the kernel that evaluates this handle's env / network: a full warp for the slot
+// kernel, the lockstep width for the GRU kernels
+static int eval_chunk(const ses_config &c)
+{
+    if (!c.gru) return 32;
+    switch (c.env) {
+    case SES_ENV_CARTPOLE: return 5;
+    case SES_ENV_MOUNTAINCAR: return GruGenConfig<MountainCarEnv>::EC;
+    case SES_ENV_ACROBOT: return GruGenConfig<AcrobotEnv>::EC;
+    case SES_ENV_PENDULUM: return GruGenConfig<PendulumEnv>::EC;
+    default: return c.n_agents == 2 ? GruGenConfig<SpreadEnv<2>>::EC : GruGenConfig<SpreadEnv<3>>::EC;
+    }
+}
+
+extern "C" int ses_evaluate(ses_handle *h, uint32_t round, const float *policies_dev, int32_t n_pol, int32_t n_episodes,
+                            const double *init_states_dev, double *returns_dev, int32_t *lengths_dev, void *stream)
+{
+    if (!h) return fail("ses_evaluate: null handle");
+    if (!policies_dev || !returns_dev || !lengths_dev) return fail("ses_evaluate: policies_dev, returns_dev and lengths_dev are required");
+    if (n_pol < 1 || n_episodes < 1) return fail("ses_evaluate: n_pol and n_episodes must be >= 1 (got %d, %d)", n_pol, n_episodes);
+    const ses_config &c = h->cfg;
+    const int E = eval_chunk(c);
+    const long long chunks = ((long long)n_episodes + E - 1) / E;
+    // the work queue counts episodes in 32-bit integers, as in ses_rollout
+    if ((long long)n_pol * chunks * E > (1ll << 30))
+        return fail("ses_evaluate: %d policies x %d episodes exceed 2^30 episodes per call", n_pol, n_episodes);
+    CU(cudaSetDevice(c.device));
+    cudaStream_t st = S(stream);
+    if (!h->eval_counter) CU(cudaMalloc(&h->eval_counter, sizeof(int) * WORK_COUNTER_INTS));
+    CU(cudaMemsetAsync(h->eval_counter, 0, sizeof(int) * WORK_COUNTER_INTS, st));
+
+    RolloutParams rp{};
+    rp.parents = policies_dev; rp.init_states = init_states_dev; rp.work_counter = h->eval_counter;
+    rp.seed = c.seed; rp.gen = round;
+    rp.init_mode = 1;                                   // counter (m, 0, round, block): Env::init with id 0 and gen = round
+    rp.layout.group = (int)chunks; rp.layout.n_head = (int)chunks; rp.layout.antithetic = 0;   // parent = policy, never perturbed
+    rp.shard.id_begin = 0; rp.shard.n_local = (int)(n_pol * chunks); rp.shard.block = 0; rp.shard.rank = 0; rp.shard.world = 1;
+    rp.E = E; rp.max_step = h->eff_max_step; rp.pomdp = c.pomdp; rp.n_agents = c.n_agents;
+    rp.sparse_rank = -1; rp.split_ok = 0;
+    rp.eval_returns = returns_dev; rp.eval_lengths = lengths_dev; rp.eval_episodes = n_episodes;
+
+    if (c.env == SES_ENV_CARTPOLE && !c.gru) return launch_eval_slots<CartpoleMlpEnvT<7>, 8>(h, rp, st);
+    if (c.env == SES_ENV_CARTPOLE) return launch_rollout_cartpole_gru_ec<5, true>(h->num_sms, h->ctas_per_sm, rp, false, st, &h->launches, g_err, sizeof(g_err));
+    if (c.gru) {
+        switch (c.env) {
+        case SES_ENV_MOUNTAINCAR: return launch_rollout_gru_generic<MountainCarEnv, true>(h->num_sms, h->ctas_per_sm, rp, false, st, &h->launches, g_err, sizeof(g_err));
+        case SES_ENV_ACROBOT: return launch_rollout_gru_generic<AcrobotEnv, true>(h->num_sms, h->ctas_per_sm, rp, false, st, &h->launches, g_err, sizeof(g_err));
+        case SES_ENV_PENDULUM: return launch_rollout_gru_generic<PendulumEnv, true>(h->num_sms, h->ctas_per_sm, rp, false, st, &h->launches, g_err, sizeof(g_err));
+        default:
+            if (c.n_agents == 2) return launch_rollout_gru_generic<SpreadEnv<2>, true>(h->num_sms, h->ctas_per_sm, rp, false, st, &h->launches, g_err, sizeof(g_err));
+            return launch_rollout_gru_generic<SpreadEnv<3>, true>(h->num_sms, h->ctas_per_sm, rp, false, st, &h->launches, g_err, sizeof(g_err));
+        }
+    }
+    if (c.env == SES_ENV_MOUNTAINCAR) return launch_eval_slots<MountainCarEnv, 8>(h, rp, st);
+    if (c.env == SES_ENV_ACROBOT) return launch_eval_slots<AcrobotEnv, 8>(h, rp, st);
+    if (c.env == SES_ENV_PENDULUM) return launch_eval_slots<PendulumEnv, 8>(h, rp, st);
+    if (c.n_agents == 2) return launch_eval_slots<SpreadEnv<2>, 6>(h, rp, st);   // shared-memory sizes as in ses_rollout
+    return launch_eval_slots<SpreadEnv<3>, 6, 2>(h, rp, st);
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -212,6 +212,28 @@ class RolloutEngine:
             return fitness, steps, trace, actions
         return fitness, steps
 
+    # ------------------------------------------------------------------------------ policy evaluation
+    def evaluate(self, policies, n_episodes, round=0, init_states=None):
+        """Run every policy ([D] or [n_pol, D] f32, used as given: no noise) for n_episodes episodes of this engine's env.
+        Episode m starts from the same state for every policy: drawn from the env's reset distribution keyed by
+        (seed, round, m), or init_states[m] ([n_episodes, state_dim] f64).  Returns (returns [n_pol, n_episodes] f64,
+        lengths [n_pol, n_episodes] i32), CUDA tensors on this engine's stream (DESIGN.md section 4.9)."""
+        if not torch.is_tensor(policies) or policies.dim() not in (1, 2) or policies.shape[-1] != self.D:
+            raise ValueError("policies has shape %s, expected [%d] or [n_pol, %d] (D of this env / network)"
+                             % (tuple(getattr(policies, "shape", ())), self.D, self.D))
+        if not (policies.is_cuda and policies.dtype == torch.float32):
+            raise ValueError("policies must be a float32 CUDA tensor")
+        policies = policies.reshape(-1, self.D).contiguous()
+        n_pol, M = policies.shape[0], int(n_episodes)
+        if M < 1:
+            raise ValueError("n_episodes must be >= 1 (got %d)" % M)
+        init_states = self._chk(init_states, torch.float64, M * self.state_dim, "init_states")
+        returns = torch.empty((n_pol, M), dtype=torch.float64, device=self.device)
+        lengths = torch.empty((n_pol, M), dtype=torch.int32, device=self.device)
+        self._check(self.lib.ses_evaluate(self._h, int(round) & 0xFFFFFFFF, _ptr(policies), n_pol, M, _ptr(init_states),
+                                          _ptr(returns), _ptr(lengths), self._stream()))
+        return returns, lengths
+
     # ------------------------------------------------------------------------------ K2
     def rank_desc(self, fitness, shaped=False, order=None, shaped_out=None, full_key=False):
         """order[r] = offspring with rank r (0 = best; ties by descending index); optional centered ranks."""

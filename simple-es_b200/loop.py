@@ -5,6 +5,11 @@ Observable behaviour kept from ESLoop: constructor signature (plus the split con
 generation print line (loop.py:89-91), wandb keys (loop.py:94-99), and
 ``logs/<env.name>/<%Y%m%d%H%M%S>/saved_models/ep_<n>.pt`` holding the elite's
 GymEnvModel-compatible state_dict every ``save_model_period`` generations (loop.py:40-47,101-104).
+
+Opt-in (``engine.eval_every: N``): after every generation ep_num with ep_num % N == 0 the policy the loop saves
+(``elite_flat()``) is evaluated on ``engine.eval_episodes`` episodes (default 100, test.py's count) keyed by ep_num, so a
+resumed run reports what the uninterrupted one does; rank 0 prints one more line, wandb gets ``eval_mean_reward`` /
+``eval_std_reward`` and ``eval_history`` one entry.  Every rank runs the same evaluation (identical results, no collective).
 """
 import os
 import time
@@ -57,6 +62,11 @@ class B200Loop(BaseESLoop):
         self.net_cfg = net_cfg
         self.strategy = STRATEGIES[strat_cfg["name"]](strat_cfg, env_cfg, net_cfg, eval_ep_num, seed, device, self.engine_cfg)
         self.history = []
+        self.eval_history = []             # (ep_num, episodes, mean, std, min, max, mean length, seconds) per evaluation
+        self.eval_every = int(self.engine_cfg.get("eval_every", 0) or 0)
+        self.eval_episodes = int(self.engine_cfg.get("eval_episodes", 100))
+        if self.eval_every < 0 or self.eval_episodes < 1:
+            raise ValueError("engine.eval_every must be >= 0 and engine.eval_episodes >= 1")
         self.start_ep = 0
         # engine.init_from: a reference-format checkpoint (GymEnvModel.state_dict(), e.g. a saved ep_<n>.pt) as the initial
         # mu / elites; engine.resume: a resume_ep_<n>.pt written by this loop (engine.save_state: true) -- continues the
@@ -87,6 +97,16 @@ class B200Loop(BaseESLoop):
         n = self.net_cfg
         return checkpoint.flat_to_state_dict(self.strategy.elite_flat(), int(n["num_state"]), int(n["num_action"]), bool(n["gru"]))
 
+    def evaluate_elite(self, ep_num):
+        """Returns of the policy elite_flat() on eval_episodes episodes keyed by ep_num: one eval_history entry."""
+        start = time.time()
+        ret, lng = self.strategy.engine.evaluate(self.strategy.elite_flat(), self.eval_episodes, round=ep_num)
+        ret, lng = ret[0].cpu(), lng[0].to(torch.float64).cpu()
+        std = float(ret.std(unbiased=False)) if ret.numel() > 1 else 0.0
+        entry = (ep_num, ret.numel(), float(ret.mean()), std, float(ret.min()), float(ret.max()), float(lng.mean()), time.time() - start)
+        self.eval_history.append(entry)
+        return entry
+
     def run(self):
         s = self.strategy
         s.timing = True                                      # CUDA-event marks around K1 + exchange and K2 + K3
@@ -113,6 +133,13 @@ class B200Loop(BaseESLoop):
                 self.ep5_rewards.append(best_reward)
                 self._wandb.log({"ep5_mean_reward": sum(self.ep5_rewards) / len(self.ep5_rewards),
                                  "curr_sigma": curr_sigma})
+            if self.eval_every and ep_num % self.eval_every == 0:
+                _, n, mean, std, lo, hi, mlen, secs = self.evaluate_elite(ep_num)
+                if self.rank == 0 and not self.quiet:
+                    print(f"  eval: {n} episodes, mean {mean:.2f}, std {std:.2f}, min {lo:.2f}, max {hi:.2f}, "
+                          f"mean length {mlen:.1f}, time: {secs:.2f}")
+                if self._wandb is not None:
+                    self._wandb.log({"eval_mean_reward": mean, "eval_std_reward": std})
             if self.rank == 0 and self.save_model_period and self.save_model_period > 0 and ep_num % self.save_model_period == 0:
                 torch.save(self.elite_state_dict(), self.save_dir + "/saved_models" + f"/ep_{ep_num}.pt")
                 if self.engine_cfg.get("save_state"):
