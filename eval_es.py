@@ -3,12 +3,18 @@
 its rendering.
 
     python eval_es.py --cfg-path conf/cartpole.yaml --ckpt-path logs/CartPole-v1/<ts>/saved_models/ep_100.pt [more.pt ...] \\
-        --episodes 100 --seed 0 [--round 0] [--out returns.npz]
+        --episodes 100 --seed 0 [--round 0] [--out returns.npz [--record K]]
 
 Each checkpoint is a GymEnvModel state_dict (ep_<n>.pt, as B200Loop and the reference save them).  All checkpoints run in
 one call on the same episodes: episode m starts from the env's reset distribution keyed by (seed, round, m), so policies are
 compared on identical initial states.  One line per checkpoint; --out writes returns [n_ckpt, episodes] (float64), lengths
 [n_ckpt, episodes] (int32) and the checkpoint paths to an .npz file.
+
+--record K also records the first K of those episodes step by step and adds them to --out: initial [K, state_dim] (the
+initial states), states [n_ckpt, K, T, state_dim] (the state after each step; for the gym envs their env.unwrapped.state, so
+a gym install can replay them into its renderer), actions [n_ckpt, K, T, n_agents], step_returns [n_ckpt, K, T] (the return
+after each step), T = the episode cap; steps past an episode's end hold NaN / -1.  The episodes' lengths are the first K
+columns of `lengths`.
 """
 import argparse
 
@@ -24,10 +30,17 @@ def parse_args(argv=None):
     ap.add_argument("--seed", type=int, default=0, help="seed of the initial states.")
     ap.add_argument("--round", type=int, default=0, help="another set of initial states under the same seed.")
     ap.add_argument("--out", default=None, help="write returns, lengths and the checkpoint paths to this .npz file.")
+    ap.add_argument("--record", type=int, default=None, metavar="K",
+                    help="also record the first K episodes step by step (states, actions, returns) into --out.")
     ap.add_argument("--device", type=int, default=0, help="CUDA device.")
     args = ap.parse_args(argv)
     if args.episodes < 1:
         ap.error("--episodes must be >= 1")
+    if args.record is not None:
+        if not args.out:
+            ap.error("--record needs --out")
+        if not 1 <= args.record <= args.episodes:
+            ap.error("--record K needs 1 <= K <= --episodes")
     if not 0 <= args.round < 2 ** 32:
         ap.error("--round must be in [0, 2^32)")
     return args
@@ -72,8 +85,12 @@ def main(argv=None):
     for path, r, n in zip(args.ckpt_path, ret, lng):
         print(f"{path}: {r.size} episodes, mean {r.mean():.2f}, std {r.std():.2f}, min {r.min():.2f}, max {r.max():.2f}, "
               f"mean length {n.mean():.1f}")
+    recorded = {}
+    if args.record:
+        rec = eng.record(W.to(eng.device), args.record, round=args.round)           # its lengths are lng[:, :K]
+        recorded = {k: t.cpu().numpy() for k, t in zip(("initial", "states", "actions", "step_returns"), rec[:4])}
     if args.out:
-        np.savez(args.out, returns=ret, lengths=lng, ckpt_paths=np.array(args.ckpt_path))
+        np.savez(args.out, returns=ret, lengths=lng, ckpt_paths=np.array(args.ckpt_path), **recorded)
     eng.close()
     return ret, lng
 

@@ -108,6 +108,21 @@ int ses_rollout(ses_handle *h, uint32_t generation, float sigma, const float *pa
 int ses_evaluate(ses_handle *h, uint32_t round, const float *policies_dev, int32_t n_pol, int32_t n_episodes,
                  const double *init_states_dev, double *returns_dev, int32_t *lengths_dev, void *stream);
 
+/* Episode recording -- what the reference's test.py shows on screen, as data (pixels stay out of scope): the same episodes
+ * as ses_evaluate (episode m does not depend on n_episodes: recording K episodes reproduces episodes 0 .. K-1 of any
+ * ses_evaluate call of the same round / init_states), with every step stored.  T = the handle's effective max_step.
+ *   initial_dev      [n_episodes][state_dim] f64: each episode's initial state in the layout of init_states rows (simple_spread:
+ *                    agent positions, then landmark positions)
+ *   states_dev       [n_pol][n_episodes][T][state_dim] f64: the state after step t + 1, laid out as ses_rollout's trace (the
+ *                    gym envs: their env.unwrapped.state; simple_spread: agent positions, then agent velocities)
+ *   actions_dev      [n_pol][n_episodes][T][n_agents] i32: the action of step t + 1 (Pendulum: the float32's bit pattern)
+ *   returns_dev      [n_pol][n_episodes][T] f64: the return after step t + 1; at t + 1 = lengths it equals ses_evaluate's return
+ *   lengths_dev      [n_pol][n_episodes] i32
+ * Rows past an episode's end are not written.  Every buffer is required; the other arguments are ses_evaluate's. */
+int ses_record(ses_handle *h, uint32_t round, const float *policies_dev, int32_t n_pol, int32_t n_episodes,
+               const double *init_states_dev, double *initial_dev, double *states_dev, int32_t *actions_dev,
+               double *returns_dev, int32_t *lengths_dev, void *stream);
+
 /* K2-- replaces np.flip(np.argsort(rewards)) (offspring_strategies.py:112,234,380) with the tie
  * order pinned to descending fitness, then DESCENDING index (== kind="stable"), and the centered
  * rank shaping (offspring_strategies.py:392-398).

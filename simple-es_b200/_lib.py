@@ -36,6 +36,7 @@ SYMBOLS = {
     "ses_destroy": (C.c_int, [_vp]),
     "ses_rollout": (C.c_int, [_vp, _u32, _f32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp]),
     "ses_evaluate": (C.c_int, [_vp, _u32, _vp, _i32, _i32, _vp, _vp, _vp, _vp]),
+    "ses_record": (C.c_int, [_vp, _u32, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "ses_rank_desc": (C.c_int, [_vp, _vp, _i32, _i32, _f64, _vp, _vp, _vp]),
     "ses_update_openai": (C.c_int, [_vp, _u32, _vp, _vp, _f64, _f64, _f64, _f64, _f64, _vp, _vp, _vp, _vp, _vp]),
     "ses_update_openai_sgd": (C.c_int, [_vp, _u32, _vp, _vp, _f64, _f64, _f64, _vp, _vp, _vp, _vp]),

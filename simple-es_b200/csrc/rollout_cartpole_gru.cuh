@@ -106,6 +106,17 @@ __device__ __forceinline__ GruLaneConsts gru_lane_consts(const float4 *small, in
     return c;
 }
 
+// recording (ses_record): state, action and return (the step count) after step nstep of episode m of policy j
+__device__ __forceinline__ void gru_record_step(const RolloutParams &p, int j, int m, int nstep, double x, double xd, double th, double thd,
+                                                int action)
+{
+    const size_t r = record_row(p, j, m, nstep - 1);
+    double *t = p.trace + r * 4;
+    t[0] = x; t[1] = xd; t[2] = th; t[3] = thd;
+    p.trace_actions[r] = action;
+    p.trace_returns[r] = (double)nstep;
+}
+
 // SPEC (the default since round 2: 4.38 ms against 4.62 ms at P = 4097 converged on a B200; SES_GRU_VARIANT=0 selects the
 // plain kernel in the test build): the
 // float64 physics leaves the serial tail of the step.  In the default kernel the <= 5 lanes that own an episode run, after
@@ -120,7 +131,8 @@ __device__ __forceinline__ GruLaneConsts gru_lane_consts(const float4 *small, in
 // One chunk of up to EC episodes (e0 .. e0 + ne - 1 of offspring `id`) stepped in lockstep by the calling warp; xh / obuf are
 // the warp's EC staging rows.  Returns the sum of the episode lengths (on every lane).
 // EVAL (ses_evaluate): `id` is the virtual offspring (policy * layout.group + chunk), e0 the chunk's first episode of the policy;
-// initial states from STREAM_EVAL, and every episode stores its return and length.
+// initial states from STREAM_EVAL, and every episode stores its return and length.  TRACE && EVAL (ses_record): every step of
+// every episode is recorded as well, by the owner lanes only (never the SPEC mirrors).
 template <int EC, bool SPEC, bool TRACE, int WREG = 0, bool EVAL = false, class Smem>
 __device__ __forceinline__ int gru_run_chunk(Smem &sm, float2 (*xh)[HID], float (*obuf)[HID + 4], const GruLaneConsts &c,
                                              const RolloutParams &p, int id, int local_idx, int e0, int ne, int lane)
@@ -141,6 +153,12 @@ __device__ __forceinline__ int gru_run_chunk(Smem &sm, float2 (*xh)[HID], float 
         } else {
             if constexpr (EVAL) cartpole_init(p.seed, 1, p.gen, 0u, (uint32_t)(e0 + ei), x, xd, th, thd, STREAM_EVAL);
             else cartpole_init(p.seed, p.init_mode, p.gen, (uint32_t)id, (uint32_t)(e0 + ei), x, xd, th, thd);
+        }
+    }
+    if constexpr (EVAL && TRACE) {                             // recording: the chunks of policy 0 store the initial states
+        if (alive && lane < EC && id < p.layout.group) {
+            double *t = p.trace_initial + (size_t)4 * (e0 + lane);
+            t[0] = x; t[1] = xd; t[2] = th; t[3] = thd;
         }
     }
     float h[EC];
@@ -261,7 +279,9 @@ __device__ __forceinline__ int gru_run_chunk(Smem &sm, float2 (*xh)[HID], float 
                 done = cartpole_step(x, xd, th, thd, action);
                 ++nstep;
                 if (nstep >= p.max_step) done = true;
-                if constexpr (TRACE) {
+                if constexpr (TRACE && EVAL) {
+                    gru_record_step(p, id / p.layout.group, e0 + lane, nstep, x, xd, th, thd, action);
+                } else if constexpr (TRACE) {
                     const int local = local_idx;
                     if (e0 + lane == 0 && local < p.n_trace && nstep <= 200) {
                         double *t = p.trace + ((size_t)local * 200 + (nstep - 1)) * 4;
@@ -282,7 +302,9 @@ __device__ __forceinline__ int gru_run_chunk(Smem &sm, float2 (*xh)[HID], float 
                 done = cdone;
                 ++nstep;
                 if (nstep >= p.max_step) done = true;
-                if constexpr (TRACE) {
+                if constexpr (TRACE && EVAL) {
+                    if (lane < EC) gru_record_step(p, id / p.layout.group, e0 + lane, nstep, x, xd, th, thd, act);
+                } else if constexpr (TRACE) {
                     const int local = local_idx;
                     if (lane < EC && e0 + lane == 0 && local < p.n_trace && nstep <= 200) {
                         double *t = p.trace + ((size_t)local * 200 + (nstep - 1)) * 4;
@@ -299,7 +321,7 @@ __device__ __forceinline__ int gru_run_chunk(Smem &sm, float2 (*xh)[HID], float 
     if constexpr (EVAL) {
         if (lane < ne) {
             const size_t at = (size_t)(id / p.layout.group) * p.eval_episodes + e0 + lane;
-            p.eval_returns[at] = (double)nstep;
+            if constexpr (!TRACE) p.eval_returns[at] = (double)nstep;   // (recording stored the returns step by step)
             p.eval_lengths[at] = nstep;
         }
     }
@@ -332,7 +354,7 @@ __global__ void __launch_bounds__(WARPS * 32, 2) k_rollout_cartpole_gru(const Ro
         const GruLaneConsts c = gru_lane_consts(sm.small, lane);
         if constexpr (EVAL) {                                      // one chunk of p.E == EC episodes, the policy's last one partial
             const int e0 = (id % p.layout.group) * p.E;
-            warp_steps += (unsigned long long)gru_run_chunk<EC, SPEC, false, WREG, true>(sm, sm.xh, sm.obuf, c, p, id, local_idx, e0,
+            warp_steps += (unsigned long long)gru_run_chunk<EC, SPEC, TRACE, WREG, true>(sm, sm.xh, sm.obuf, c, p, id, local_idx, e0,
                                                                                           min(p.E, p.eval_episodes - e0), lane);
             continue;
         }
@@ -460,7 +482,8 @@ static int launch_rollout_cartpole_gru_ec(int num_sms, int ctas_per_sm, const Ro
 #else
     kern = trace ? k_rollout_cartpole_gru<EC, WARPS, true, true, 1> : k_rollout_cartpole_gru<EC, WARPS, false, true, 1>;
 #endif
-    if constexpr (EVAL) kern = k_rollout_cartpole_gru<EC, WARPS, false, true, 1, true>;      // the product's kernel, evaluation instance
+    if constexpr (EVAL)                                                // the product's kernel, evaluation / recording instance
+        kern = trace ? k_rollout_cartpole_gru<EC, WARPS, true, true, 1, true> : k_rollout_cartpole_gru<EC, WARPS, false, true, 1, true>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     int per_sm = 0;
     if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, WARPS * 32, smem);

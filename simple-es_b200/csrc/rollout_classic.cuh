@@ -171,6 +171,7 @@ struct MountainCarEnv {
     }
 
     __device__ static __forceinline__ void store_trace(const State &s, double *row) { row[0] = s.pos; row[1] = s.vel; }
+    __device__ static __forceinline__ void store_init(const State &s, double *row) { store_trace(s, row); }
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -245,6 +246,7 @@ struct PendulumEnv {
     }
 
     __device__ static __forceinline__ void store_trace(const State &s, double *row) { row[0] = s.th; row[1] = s.thd; }
+    __device__ static __forceinline__ void store_init(const State &s, double *row) { store_trace(s, row); }
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -364,6 +366,7 @@ struct AcrobotEnv {
     {
         row[0] = st.s[0]; row[1] = st.s[1]; row[2] = st.s[2]; row[3] = st.s[3];
     }
+    __device__ static __forceinline__ void store_init(const State &st, double *row) { store_trace(st, row); }
 };
 
 }  // namespace ses

@@ -91,6 +91,7 @@ __device__ __forceinline__ float fc2_row_blocks(const float *w, const float *x, 
 
 // EVAL (ses_evaluate): one chunk of p.E == EC episodes per virtual offspring (policy * layout.group + chunk), the policy's last
 // chunk partial; initial states from STREAM_EVAL, and every episode stores its return and length instead of a fitness.
+// TRACE && EVAL (ses_record): every step of every episode is recorded as well (record_step; the owner lanes write).
 template <class Env, int EC, int WARPS, bool TRACE, bool EVAL = false>
 __global__ void __launch_bounds__(WARPS * 32) k_rollout_gru_generic(const RolloutParams p)
 {
@@ -136,11 +137,17 @@ __global__ void __launch_bounds__(WARPS * 32) k_rollout_gru_generic(const Rollou
             typename Env::State st;                                    // lane e < ne: episode e0 + e (other lanes: a harmless copy)
             if constexpr (EVAL) Env::template init<STREAM_EVAL>(st, p, 0, m0 + (lane < ne ? lane : 0));
             else Env::init(st, p, id, e0 + (lane < ne ? lane : 0));
+            if constexpr (EVAL && TRACE) {                             // recording: the chunks of policy 0 store the initial states
+                if (lane < ne && id < p.layout.group) Env::store_init(st, p.trace_initial + (size_t)(m0 + lane) * Env::STATE_DIM);
+            }
             bool alive = lane < ne;
             int nstep = 0;
             float h[V];
 #pragma unroll
             for (int v = 0; v < V; ++v) { h[v] = 0.0f; sm.xh[v][lane] = make_float2(0.0f, 0.0f); }      // model.reset() per agent copy
+            // recording: row of this lane's episode (computed once: inside the loop the Acrobot instance spilled 32 B instead of 8)
+            [[maybe_unused]] size_t rec = 0;
+            if constexpr (EVAL && TRACE) rec = record_row(p, id / p.layout.group, m0 + lane, 0);
             unsigned alive_mask = __ballot_sync(FULL, alive);
             while (alive_mask) {
                 // observations of every agent of every episode
@@ -226,7 +233,9 @@ __global__ void __launch_bounds__(WARPS * 32) k_rollout_gru_generic(const Rollou
                     bool done = Env::advance(st, actions);
                     ++nstep;
                     if (nstep >= p.max_step) done = true;
-                    if constexpr (TRACE) {
+                    if constexpr (TRACE && EVAL) {
+                        record_step<Env>(p, st, actions, rec + (nstep - 1), nstep);
+                    } else if constexpr (TRACE) {
                         if (e0 + lane == 0 && local_idx < p.n_trace && nstep <= 200) {
                             Env::store_trace(st, p.trace + ((size_t)local_idx * 200 + (nstep - 1)) * Env::STATE_DIM);
 #pragma unroll
@@ -240,7 +249,7 @@ __global__ void __launch_bounds__(WARPS * 32) k_rollout_gru_generic(const Rollou
             if constexpr (EVAL) {
                 if (lane < ne) {
                     const size_t at = (size_t)(id / p.layout.group) * p.eval_episodes + m0 + lane;
-                    p.eval_returns[at] = st.ret;
+                    if constexpr (!TRACE) p.eval_returns[at] = st.ret;     // (recording stored the returns step by step)
                     p.eval_lengths[at] = nstep;
                 }
             }
@@ -278,7 +287,7 @@ static int launch_rollout_gru_generic(int num_sms, int ctas_per_sm, const Rollou
 {
     constexpr int EC = GruGenConfig<Env>::EC, WARPS = GruGenConfig<Env>::WARPS;
     const size_t smem = WARPS * sizeof(GruGenSmem<Env, EC>);
-    auto kern = EVAL ? k_rollout_gru_generic<Env, EC, WARPS, false, true>
+    auto kern = EVAL ? (trace ? k_rollout_gru_generic<Env, EC, WARPS, true, true> : k_rollout_gru_generic<Env, EC, WARPS, false, true>)
               : trace ? k_rollout_gru_generic<Env, EC, WARPS, true> : k_rollout_gru_generic<Env, EC, WARPS, false>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     int per_sm = 0;

@@ -333,6 +333,16 @@ struct SpreadEnv {
             row[2 * N + 2 * i] = s.avel[i][0]; row[2 * N + 2 * i + 1] = s.avel[i][1];
         }
     }
+
+    // init_states layout: agent positions, then landmark positions (the velocities start at 0)
+    __device__ static __forceinline__ void store_init(const State &s, double *row)
+    {
+#pragma unroll
+        for (int i = 0; i < N; ++i) {
+            row[2 * i] = s.apos[i][0]; row[2 * i + 1] = s.apos[i][1];
+            row[2 * N + 2 * i] = s.lpos[i][0]; row[2 * N + 2 * i + 1] = s.lpos[i][1];
+        }
+    }
 };
 
 }  // namespace ses

@@ -30,6 +30,7 @@
 //   bind<S>(State&, w[NQ][S], slot)          a lane was handed an episode of `slot` (an Env may cache weights in registers)
 //   step<S>(State&, w[NQ][S], slot, p, int *actions) -> done   (also adds the step reward to State::ret)
 //   store_trace(State&, double *row)
+//   store_init(State&, double *row)          the initial state in the layout of init_states rows (recording)
 #pragma once
 #include "ses_common.cuh"
 
@@ -94,7 +95,29 @@ struct RolloutParams {
     double *eval_returns;        // [n_pol][eval_episodes] return of every episode
     int *eval_lengths;           // [n_pol][eval_episodes] its env steps
     int eval_episodes;
+    // recording (the TRACE && EVAL instances, ses_record): every step of every episode; trace / trace_actions are then
+    // [n_pol][eval_episodes][max_step][state_dim | n_agents] and eval_returns is unused
+    double *trace_returns;       // [n_pol][eval_episodes][max_step] return after each step
+    double *trace_initial;       // [eval_episodes][state_dim] initial states (layout of init_states rows), written by policy 0
 };
+
+// row of (episode m of policy j, step t) in the recording buffers: 64-bit, n_pol * eval_episodes * max_step * state_dim
+// passes 2^31 quickly
+__device__ __forceinline__ size_t record_row(const RolloutParams &p, int j, int m, int t)
+{
+    return ((size_t)j * p.eval_episodes + m) * p.max_step + t;
+}
+
+// recording: the state, actions and return after step `nstep`, at row r of the recording buffers
+template <class Env>
+__device__ __forceinline__ void record_step(const RolloutParams &p, const typename Env::State &st, const int *actions, size_t r, int nstep)
+{
+    Env::store_trace(st, p.trace + r * Env::STATE_DIM);
+#pragma unroll
+    for (int a = 0; a < Env::N_AGENTS; ++a) p.trace_actions[r * Env::N_AGENTS + a] = actions[a];
+    if constexpr (Env::UNIT_REWARD) p.trace_returns[r] = (double)nstep;
+    else p.trace_returns[r] = st.ret;
+}
 
 constexpr int MAX_E = 32;
 
@@ -442,6 +465,10 @@ __global__ void __launch_bounds__(WARPS * 32) k_rollout_slots(const RolloutParam
                 slot = my_slot; ep = my_ep; nstep = 0;
                 if constexpr (EVAL) Env::template init<STREAM_EVAL>(st, p, 0, (sm.off_id[my_slot] % p.layout.group) * p.E + my_ep);
                 else Env::init(st, p, sm.off_id[my_slot], my_ep);
+                if constexpr (EVAL && TRACE) {                      // recording: the chunks of policy 0 store the initial states
+                    const int vid = sm.off_id[my_slot];
+                    if (vid < p.layout.group) Env::store_init(st, p.trace_initial + (size_t)(vid * p.E + my_ep) * Env::STATE_DIM);
+                }
                 Env::template bind<S>(st, sm.w, my_slot);
             }
             __syncwarp();
@@ -463,7 +490,10 @@ __global__ void __launch_bounds__(WARPS * 32) k_rollout_slots(const RolloutParam
             bool done = Env::template step<S>(st, sm.w, slot, p, actions);
             ++nstep;                                               // gym_wrapper.py:33 / pettingzoo_wrapper.py:34
             if (nstep >= p.max_step) done = true;                  // gym_wrapper.py:37-39, TimeLimit / max_cycles
-            if constexpr (TRACE) {
+            if constexpr (TRACE && EVAL) {
+                const int vid = sm.off_id[slot];
+                record_step<Env>(p, st, actions, record_row(p, vid / p.layout.group, (vid % p.layout.group) * p.E + ep, nstep - 1), nstep);
+            } else if constexpr (TRACE) {
                 const int local = p.shard.id_to_local(sm.off_id[slot]);
                 if (ep == 0 && local < p.n_trace && nstep <= 200) {
                     Env::store_trace(st, p.trace + ((size_t)local * 200 + (nstep - 1)) * Env::STATE_DIM);
@@ -475,8 +505,10 @@ __global__ void __launch_bounds__(WARPS * 32) k_rollout_slots(const RolloutParam
                 if constexpr (EVAL) {
                     const int vid = sm.off_id[slot];
                     const size_t at = (size_t)(vid / p.layout.group) * p.eval_episodes + (vid % p.layout.group) * p.E + ep;
-                    if constexpr (Env::UNIT_REWARD) p.eval_returns[at] = (double)nstep;
-                    else p.eval_returns[at] = st.ret;
+                    if constexpr (!TRACE) {                         // (recording stored the returns step by step)
+                        if constexpr (Env::UNIT_REWARD) p.eval_returns[at] = (double)nstep;
+                        else p.eval_returns[at] = st.ret;
+                    }
                     p.eval_lengths[at] = nstep;
                 } else if constexpr (!Env::UNIT_REWARD) {
                     sm.ret[slot][ep] = st.ret;

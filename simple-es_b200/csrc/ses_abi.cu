@@ -109,7 +109,7 @@ struct ses_handle {
     int spread_slots8 = 0;
     int k1_split = 1;
     int k1_sparse = 1;
-    int *eval_counter = nullptr;   // work counter of ses_evaluate's launches (allocated by the first call)
+    int *eval_counter = nullptr;   // work counter of ses_evaluate / ses_record launches (allocated by the first call)
 
     int64_t launches = 0;
 };
@@ -463,15 +463,15 @@ extern "C" int ses_rollout(ses_handle *h, uint32_t generation, float sigma, cons
 }
 
 // ------------------------------------------------------------------------------------------------
-// policy evaluation (DESIGN.md section 4.9): the EVAL instances of the K1 kernels
+// policy evaluation and recording (DESIGN.md section 4.9): the EVAL and TRACE && EVAL instances of the K1 kernels
 // ------------------------------------------------------------------------------------------------
 // The slot kernel with chunks of E = 32 episodes: one chunk fills a warp.  Whole chunks only (queue A), so a chunk's clipped
-// episode count is exact; no sparse warps, no straggler phase.
+// episode count is exact; no sparse warps, no straggler phase.  `record`: the TRACE instance (ses_record).
 template <class Env, int SL, int WARPS = 4>
-static int launch_eval_slots(ses_handle *h, RolloutParams &rp, cudaStream_t st)
+static int launch_eval_slots(ses_handle *h, RolloutParams &rp, bool record, cudaStream_t st)
 {
     using Smem = SlotSmem<Env, SL, !Env::UNIT_REWARD>;
-    auto kernel = k_rollout_slots<Env, SL, WARPS, false, false, true>;
+    auto kernel = record ? k_rollout_slots<Env, SL, WARPS, true, false, true> : k_rollout_slots<Env, SL, WARPS, false, false, true>;
     const size_t smem = WARPS * sizeof(Smem);
     CU(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 0;
@@ -503,24 +503,23 @@ static int eval_chunk(const ses_config &c)
     }
 }
 
-extern "C" int ses_evaluate(ses_handle *h, uint32_t round, const float *policies_dev, int32_t n_pol, int32_t n_episodes,
-                            const double *init_states_dev, double *returns_dev, int32_t *lengths_dev, void *stream)
+// The launch of ses_evaluate and ses_record: n_pol x n_episodes episodes as virtual offspring (policy, chunk).  rp carries
+// the caller's output pointers; `record` selects the TRACE instance of each kernel family.
+static int launch_eval(ses_handle *h, const char *fn, uint32_t round, const float *policies_dev, int32_t n_pol, int32_t n_episodes,
+                       const double *init_states_dev, RolloutParams &rp, bool record, void *stream)
 {
-    if (!h) return fail("ses_evaluate: null handle");
-    if (!policies_dev || !returns_dev || !lengths_dev) return fail("ses_evaluate: policies_dev, returns_dev and lengths_dev are required");
-    if (n_pol < 1 || n_episodes < 1) return fail("ses_evaluate: n_pol and n_episodes must be >= 1 (got %d, %d)", n_pol, n_episodes);
+    if (n_pol < 1 || n_episodes < 1) return fail("%s: n_pol and n_episodes must be >= 1 (got %d, %d)", fn, n_pol, n_episodes);
     const ses_config &c = h->cfg;
     const int E = eval_chunk(c);
     const long long chunks = ((long long)n_episodes + E - 1) / E;
     // the work queue counts episodes in 32-bit integers, as in ses_rollout
     if ((long long)n_pol * chunks * E > (1ll << 30))
-        return fail("ses_evaluate: %d policies x %d episodes exceed 2^30 episodes per call", n_pol, n_episodes);
+        return fail("%s: %d policies x %d episodes exceed 2^30 episodes per call", fn, n_pol, n_episodes);
     CU(cudaSetDevice(c.device));
     cudaStream_t st = S(stream);
     if (!h->eval_counter) CU(cudaMalloc(&h->eval_counter, sizeof(int) * WORK_COUNTER_INTS));
     CU(cudaMemsetAsync(h->eval_counter, 0, sizeof(int) * WORK_COUNTER_INTS, st));
 
-    RolloutParams rp{};
     rp.parents = policies_dev; rp.init_states = init_states_dev; rp.work_counter = h->eval_counter;
     rp.seed = c.seed; rp.gen = round;
     rp.init_mode = 1;                                   // counter (m, 0, round, block): Env::init with id 0 and gen = round
@@ -528,25 +527,48 @@ extern "C" int ses_evaluate(ses_handle *h, uint32_t round, const float *policies
     rp.shard.id_begin = 0; rp.shard.n_local = (int)(n_pol * chunks); rp.shard.block = 0; rp.shard.rank = 0; rp.shard.world = 1;
     rp.E = E; rp.max_step = h->eff_max_step; rp.pomdp = c.pomdp; rp.n_agents = c.n_agents;
     rp.sparse_rank = -1; rp.split_ok = 0;
-    rp.eval_returns = returns_dev; rp.eval_lengths = lengths_dev; rp.eval_episodes = n_episodes;
+    rp.eval_episodes = n_episodes;
 
-    if (c.env == SES_ENV_CARTPOLE && !c.gru) return launch_eval_slots<CartpoleMlpEnvT<7>, 8>(h, rp, st);
-    if (c.env == SES_ENV_CARTPOLE) return launch_rollout_cartpole_gru_ec<5, true>(h->num_sms, h->ctas_per_sm, rp, false, st, &h->launches, g_err, sizeof(g_err));
+    if (c.env == SES_ENV_CARTPOLE && !c.gru) return launch_eval_slots<CartpoleMlpEnvT<7>, 8>(h, rp, record, st);
+    if (c.env == SES_ENV_CARTPOLE) return launch_rollout_cartpole_gru_ec<5, true>(h->num_sms, h->ctas_per_sm, rp, record, st, &h->launches, g_err, sizeof(g_err));
     if (c.gru) {
         switch (c.env) {
-        case SES_ENV_MOUNTAINCAR: return launch_rollout_gru_generic<MountainCarEnv, true>(h->num_sms, h->ctas_per_sm, rp, false, st, &h->launches, g_err, sizeof(g_err));
-        case SES_ENV_ACROBOT: return launch_rollout_gru_generic<AcrobotEnv, true>(h->num_sms, h->ctas_per_sm, rp, false, st, &h->launches, g_err, sizeof(g_err));
-        case SES_ENV_PENDULUM: return launch_rollout_gru_generic<PendulumEnv, true>(h->num_sms, h->ctas_per_sm, rp, false, st, &h->launches, g_err, sizeof(g_err));
+        case SES_ENV_MOUNTAINCAR: return launch_rollout_gru_generic<MountainCarEnv, true>(h->num_sms, h->ctas_per_sm, rp, record, st, &h->launches, g_err, sizeof(g_err));
+        case SES_ENV_ACROBOT: return launch_rollout_gru_generic<AcrobotEnv, true>(h->num_sms, h->ctas_per_sm, rp, record, st, &h->launches, g_err, sizeof(g_err));
+        case SES_ENV_PENDULUM: return launch_rollout_gru_generic<PendulumEnv, true>(h->num_sms, h->ctas_per_sm, rp, record, st, &h->launches, g_err, sizeof(g_err));
         default:
-            if (c.n_agents == 2) return launch_rollout_gru_generic<SpreadEnv<2>, true>(h->num_sms, h->ctas_per_sm, rp, false, st, &h->launches, g_err, sizeof(g_err));
-            return launch_rollout_gru_generic<SpreadEnv<3>, true>(h->num_sms, h->ctas_per_sm, rp, false, st, &h->launches, g_err, sizeof(g_err));
+            if (c.n_agents == 2) return launch_rollout_gru_generic<SpreadEnv<2>, true>(h->num_sms, h->ctas_per_sm, rp, record, st, &h->launches, g_err, sizeof(g_err));
+            return launch_rollout_gru_generic<SpreadEnv<3>, true>(h->num_sms, h->ctas_per_sm, rp, record, st, &h->launches, g_err, sizeof(g_err));
         }
     }
-    if (c.env == SES_ENV_MOUNTAINCAR) return launch_eval_slots<MountainCarEnv, 8>(h, rp, st);
-    if (c.env == SES_ENV_ACROBOT) return launch_eval_slots<AcrobotEnv, 8>(h, rp, st);
-    if (c.env == SES_ENV_PENDULUM) return launch_eval_slots<PendulumEnv, 8>(h, rp, st);
-    if (c.n_agents == 2) return launch_eval_slots<SpreadEnv<2>, 6>(h, rp, st);   // shared-memory sizes as in ses_rollout
-    return launch_eval_slots<SpreadEnv<3>, 6, 2>(h, rp, st);
+    if (c.env == SES_ENV_MOUNTAINCAR) return launch_eval_slots<MountainCarEnv, 8>(h, rp, record, st);
+    if (c.env == SES_ENV_ACROBOT) return launch_eval_slots<AcrobotEnv, 8>(h, rp, record, st);
+    if (c.env == SES_ENV_PENDULUM) return launch_eval_slots<PendulumEnv, 8>(h, rp, record, st);
+    if (c.n_agents == 2) return launch_eval_slots<SpreadEnv<2>, 6>(h, rp, record, st);   // shared-memory sizes as in ses_rollout
+    return launch_eval_slots<SpreadEnv<3>, 6, 2>(h, rp, record, st);
+}
+
+extern "C" int ses_evaluate(ses_handle *h, uint32_t round, const float *policies_dev, int32_t n_pol, int32_t n_episodes,
+                            const double *init_states_dev, double *returns_dev, int32_t *lengths_dev, void *stream)
+{
+    if (!h) return fail("ses_evaluate: null handle");
+    if (!policies_dev || !returns_dev || !lengths_dev) return fail("ses_evaluate: policies_dev, returns_dev and lengths_dev are required");
+    RolloutParams rp{};
+    rp.eval_returns = returns_dev; rp.eval_lengths = lengths_dev;
+    return launch_eval(h, "ses_evaluate", round, policies_dev, n_pol, n_episodes, init_states_dev, rp, false, stream);
+}
+
+extern "C" int ses_record(ses_handle *h, uint32_t round, const float *policies_dev, int32_t n_pol, int32_t n_episodes,
+                          const double *init_states_dev, double *initial_dev, double *states_dev, int32_t *actions_dev,
+                          double *returns_dev, int32_t *lengths_dev, void *stream)
+{
+    if (!h) return fail("ses_record: null handle");
+    if (!policies_dev || !initial_dev || !states_dev || !actions_dev || !returns_dev || !lengths_dev)
+        return fail("ses_record: policies_dev, initial_dev, states_dev, actions_dev, returns_dev and lengths_dev are required");
+    RolloutParams rp{};
+    rp.trace_initial = initial_dev; rp.trace = states_dev; rp.trace_actions = actions_dev; rp.trace_returns = returns_dev;
+    rp.eval_lengths = lengths_dev;
+    return launch_eval(h, "ses_record", round, policies_dev, n_pol, n_episodes, init_states_dev, rp, true, stream);
 }
 
 // ------------------------------------------------------------------------------------------------

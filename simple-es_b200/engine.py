@@ -234,6 +234,39 @@ class RolloutEngine:
                                           _ptr(returns), _ptr(lengths), self._stream()))
         return returns, lengths
 
+    def record(self, policies, n_episodes, round=0, init_states=None):
+        """Record, step by step, episodes 0 .. n_episodes-1 of what `evaluate` runs with the same round / init_states (episode m
+        does not depend on the episode count).  Returns, as CUDA tensors on this engine's stream, with K = n_episodes and
+        T = max_step (DESIGN.md section 4.9):
+          initial [K, state_dim] f64            the initial states, laid out as init_states rows
+          states  [n_pol, K, T, state_dim] f64  the state after step t + 1 (gym envs: env.unwrapped.state; simple_spread:
+                                                agent positions, then agent velocities)
+          actions [n_pol, K, T, n_agents] i32   the action of step t + 1; float32 for continuous-action envs
+          returns [n_pol, K, T] f64             the return after step t + 1: returns[j, m, lengths[j, m] - 1] is evaluate's
+          lengths [n_pol, K] i32
+        Steps past an episode's end hold NaN (actions: -1, or NaN for float32 actions)."""
+        if not torch.is_tensor(policies) or policies.dim() not in (1, 2) or policies.shape[-1] != self.D:
+            raise ValueError("policies has shape %s, expected [%d] or [n_pol, %d] (D of this env / network)"
+                             % (tuple(getattr(policies, "shape", ())), self.D, self.D))
+        if not (policies.is_cuda and policies.dtype == torch.float32):
+            raise ValueError("policies must be a float32 CUDA tensor")
+        policies = policies.reshape(-1, self.D).contiguous()
+        n_pol, K, T = policies.shape[0], int(n_episodes), self.max_step
+        if K < 1:
+            raise ValueError("n_episodes must be >= 1 (got %d)" % K)
+        init_states = self._chk(init_states, torch.float64, K * self.state_dim, "init_states")
+        dev, nan = self.device, float("nan")
+        initial = torch.full((K, self.state_dim), nan, dtype=torch.float64, device=dev)
+        states = torch.full((n_pol, K, T, self.state_dim), nan, dtype=torch.float64, device=dev)
+        actions = torch.full((n_pol, K, T, self.n_agents), -1, dtype=torch.int32, device=dev)
+        returns = torch.full((n_pol, K, T), nan, dtype=torch.float64, device=dev)
+        lengths = torch.full((n_pol, K), -1, dtype=torch.int32, device=dev)
+        self._check(self.lib.ses_record(self._h, int(round) & 0xFFFFFFFF, _ptr(policies), n_pol, K, _ptr(init_states),
+                                        _ptr(initial), _ptr(states), _ptr(actions), _ptr(returns), _ptr(lengths), self._stream()))
+        if self.env_name in CONTINUOUS_ENVS:
+            actions = actions.view(torch.float32)
+        return initial, states, actions, returns, lengths
+
     # ------------------------------------------------------------------------------ K2
     def rank_desc(self, fitness, shaped=False, order=None, shaped_out=None, full_key=False):
         """order[r] = offspring with rank r (0 = best; ties by descending index); optional centered ranks."""
