@@ -205,6 +205,27 @@ int ses_measure_fp32x2_peak(int32_t device, double *tflops_out);
 /* Optional device counter (uint64): every ses_rollout adds the env steps it simulated (bench.py's numerator). */
 int ses_set_step_counter(ses_handle *h, uint64_t *counter_dev);
 
+/* Optional device buffer [population][eval_ep_num][state_dim] f64 (NULL: off, the default).  While set, every ses_rollout also
+ * stores the state after each episode's last step at row (global offspring id) * eval_ep_num + episode, in the layout of
+ * ses_record's states (the gym envs: env.unwrapped.state; simple_spread: agent positions, then agent velocities).  Only the
+ * rows of the ids this handle owns are written; fitness and steps are the same as without it.  ses_rollout then refuses
+ * n_trace > 0.  ses_evaluate and ses_record ignore it. */
+int ses_set_final_states(ses_handle *h, double *final_states_dev);
+
+/* Novelty search with reward (the nsr_es strategy, DESIGN.md section 4.10).  float64 throughout, each operation separately
+ * rounded; every call is stream-ordered and runs on the handle's device.  1 <= n <= population.
+ * ses_behavior:     bc_dev[i][d] = (sum over e in episode order of final_states_dev[i][e][d]) / eval_ep_num, i < n
+ * ses_novelty:      novelty_dev[i] = mean of the Euclidean distances sqrt(sum_d (bc[i][d] - archive[a][d])^2) from bc_dev[i] to
+ *                   its min(k, n_archive) nearest rows of archive_dev [n_archive][state_dim], added in ascending order;
+ *                   1 <= k <= 32, n_archive >= 1
+ * ses_blend_shaped: out_dev[i] = (1 - w) shaped_f_dev[i] + w shaped_n_dev[i], 0 <= w <= 1 (w = 0 returns shaped_f_dev's
+ *                   values, w = 1 shaped_n_dev's, for any shaping without -0.0 entries such as ses_rank_desc's) */
+int ses_behavior(ses_handle *h, const double *final_states_dev, int32_t n, double *bc_dev, void *stream);
+int ses_novelty(ses_handle *h, const double *bc_dev, int32_t n, const double *archive_dev, int32_t n_archive, int32_t k,
+                double *novelty_dev, void *stream);
+int ses_blend_shaped(ses_handle *h, const double *shaped_f_dev, const double *shaped_n_dev, int32_t n, double w, double *out_dev,
+                     void *stream);
+
 /* Number of kernels this library has launched on behalf of the handle (bench.py "gpu_launches"). */
 int64_t ses_launch_count(ses_handle *h);
 

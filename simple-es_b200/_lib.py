@@ -13,7 +13,7 @@ TEST_LIB_PATH = os.path.join(_PKG, "libses_b200_tests.so")
 SOURCES = [os.path.join(_PKG, "csrc", f) for f in (
     "ses_abi.cu", "ses_common.cuh", "rollout_slots.cuh", "rollout_cartpole_mlp.cuh", "rollout_cartpole_gru.cuh", "rollout_mpe.cuh",
     "rollout_classic.cuh", "rollout_gru_generic.cuh",
-    "rank.cuh", "update.cuh")]
+    "rank.cuh", "update.cuh", "novelty.cuh")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-fmad=false",           # numerical contract: FMAs only where written (DESIGN.md section 4)
               "-Xcompiler", "-fPIC", "-shared"]
@@ -54,6 +54,10 @@ SYMBOLS = {
     "ses_measure_fp32x2_peak": (C.c_int, [_i32, C.POINTER(C.c_double)]),
     "ses_set_step_counter": (C.c_int, [_vp, _vp]),
     "ses_launch_count": (_i64, [_vp]),
+    "ses_set_final_states": (C.c_int, [_vp, _vp]),
+    "ses_behavior": (C.c_int, [_vp, _vp, _i32, _vp, _vp]),
+    "ses_novelty": (C.c_int, [_vp, _vp, _i32, _vp, _i32, _i32, _vp, _vp]),
+    "ses_blend_shaped": (C.c_int, [_vp, _vp, _vp, _i32, _f64, _vp, _vp]),
 }
 # include/ses_b200_test.h: only in the test build
 TEST_SYMBOLS = {

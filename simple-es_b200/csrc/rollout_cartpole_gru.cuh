@@ -132,8 +132,9 @@ __device__ __forceinline__ void gru_record_step(const RolloutParams &p, int j, i
 // the warp's EC staging rows.  Returns the sum of the episode lengths (on every lane).
 // EVAL (ses_evaluate): `id` is the virtual offspring (policy * layout.group + chunk), e0 the chunk's first episode of the policy;
 // initial states from STREAM_EVAL, and every episode stores its return and length.  TRACE && EVAL (ses_record): every step of
-// every episode is recorded as well, by the owner lanes only (never the SPEC mirrors).
-template <int EC, bool SPEC, bool TRACE, int WREG = 0, bool EVAL = false, class Smem>
+// every episode is recorded as well, by the owner lanes only (never the SPEC mirrors).  FINAL (training, ses_set_final_states):
+// the owner lanes store each episode's final state.
+template <int EC, bool SPEC, bool TRACE, int WREG = 0, bool EVAL = false, bool FINAL = false, class Smem>
 __device__ __forceinline__ int gru_run_chunk(Smem &sm, float2 (*xh)[HID], float (*obuf)[HID + 4], const GruLaneConsts &c,
                                              const RolloutParams &p, int id, int local_idx, int e0, int ne, int lane)
 {
@@ -317,6 +318,12 @@ __device__ __forceinline__ int gru_run_chunk(Smem &sm, float2 (*xh)[HID], float 
         }
         alive_mask = __ballot_sync(FULL, alive);
     }
+    if constexpr (FINAL) {
+        if (lane < ne) {                                       // lanes < ne <= EC: the owners, never a SPEC mirror
+            double *row = final_row(p, id, e0 + lane, 4);
+            row[0] = x; row[1] = xd; row[2] = th; row[3] = thd;
+        }
+    }
     // chunk total: lanes 0..ne-1 hold their episode lengths
     if constexpr (EVAL) {
         if (lane < ne) {
@@ -331,7 +338,7 @@ __device__ __forceinline__ int gru_run_chunk(Smem &sm, float2 (*xh)[HID], float 
     return n;
 }
 
-template <int EC, int WARPS, bool TRACE, bool SPEC = false, int WREG = 0, bool EVAL = false>
+template <int EC, int WARPS, bool TRACE, bool SPEC = false, int WREG = 0, bool EVAL = false, bool FINAL = false>
 __global__ void __launch_bounds__(WARPS * 32, 2) k_rollout_cartpole_gru(const RolloutParams p)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -360,7 +367,7 @@ __global__ void __launch_bounds__(WARPS * 32, 2) k_rollout_cartpole_gru(const Ro
         }
         long long total_steps = 0;
         for (int e0 = 0; e0 < p.E; e0 += EC)
-            total_steps += gru_run_chunk<EC, SPEC, TRACE, WREG>(sm, sm.xh, sm.obuf, c, p, id, local_idx, e0, min(EC, p.E - e0), lane);
+            total_steps += gru_run_chunk<EC, SPEC, TRACE, WREG, false, FINAL>(sm, sm.xh, sm.obuf, c, p, id, local_idx, e0, min(EC, p.E - e0), lane);
         warp_steps += (unsigned long long)total_steps;
         if (lane == 0) {
             p.steps[id] = total_steps;
@@ -464,7 +471,7 @@ static int launch_rollout_cartpole_gru_pair(int num_sms, int ctas_per_sm, const 
 
 template <int EC, bool EVAL = false>
 static int launch_rollout_cartpole_gru_ec(int num_sms, int ctas_per_sm, const RolloutParams &rp, bool trace, cudaStream_t st,
-                                          int64_t *launches, char *err, size_t errlen)
+                                          int64_t *launches, char *err, size_t errlen, bool final_states = false)
 {
     constexpr int WARPS = 4;
     const size_t smem = WARPS * sizeof(GruWarpSmem<EC>);
@@ -484,6 +491,8 @@ static int launch_rollout_cartpole_gru_ec(int num_sms, int ctas_per_sm, const Ro
 #endif
     if constexpr (EVAL)                                                // the product's kernel, evaluation / recording instance
         kern = trace ? k_rollout_cartpole_gru<EC, WARPS, true, true, 1, true> : k_rollout_cartpole_gru<EC, WARPS, false, true, 1, true>;
+    else if (final_states)                                             // the product's kernel, final-state instance
+        kern = k_rollout_cartpole_gru<EC, WARPS, false, true, 1, false, true>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     int per_sm = 0;
     if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, WARPS * 32, smem);
@@ -506,6 +515,15 @@ static int launch_rollout_cartpole_gru_ec(int num_sms, int ctas_per_sm, const Ro
 static int launch_rollout_cartpole_gru(int num_sms, int ctas_per_sm, const RolloutParams &rp, bool trace, cudaStream_t st,
                                        int64_t *launches, char *err, size_t errlen)
 {
+    if (rp.final_states) {                                             // the product's kernel with the final-state output
+        switch (rp.E >= 5 ? 5 : rp.E) {
+        case 1: return launch_rollout_cartpole_gru_ec<1>(num_sms, ctas_per_sm, rp, false, st, launches, err, errlen, true);
+        case 2: return launch_rollout_cartpole_gru_ec<2>(num_sms, ctas_per_sm, rp, false, st, launches, err, errlen, true);
+        case 3: return launch_rollout_cartpole_gru_ec<3>(num_sms, ctas_per_sm, rp, false, st, launches, err, errlen, true);
+        case 4: return launch_rollout_cartpole_gru_ec<4>(num_sms, ctas_per_sm, rp, false, st, launches, err, errlen, true);
+        default: return launch_rollout_cartpole_gru_ec<5>(num_sms, ctas_per_sm, rp, false, st, launches, err, errlen, true);
+        }
+    }
     // episodes of one offspring step in lockstep, EC at a time (E > 5: chunks of 5, the last one partial)
 #ifdef SES_BUILD_TESTS
     {   // SES_GRU_VARIANT=2: the warp-pair kernel (rejected: 5.48 ms against 4.30 ms, profiles/r02_k1_experiments.md)

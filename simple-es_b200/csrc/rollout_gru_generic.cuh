@@ -92,7 +92,8 @@ __device__ __forceinline__ float fc2_row_blocks(const float *w, const float *x, 
 // EVAL (ses_evaluate): one chunk of p.E == EC episodes per virtual offspring (policy * layout.group + chunk), the policy's last
 // chunk partial; initial states from STREAM_EVAL, and every episode stores its return and length instead of a fitness.
 // TRACE && EVAL (ses_record): every step of every episode is recorded as well (record_step; the owner lanes write).
-template <class Env, int EC, int WARPS, bool TRACE, bool EVAL = false>
+// FINAL (training, ses_set_final_states): the owner lanes store each episode's final state.
+template <class Env, int EC, int WARPS, bool TRACE, bool EVAL = false, bool FINAL = false>
 __global__ void __launch_bounds__(WARPS * 32) k_rollout_gru_generic(const RolloutParams p)
 {
     using Smem = GruGenSmem<Env, EC>;
@@ -246,6 +247,9 @@ __global__ void __launch_bounds__(WARPS * 32) k_rollout_gru_generic(const Rollou
                 }
                 alive_mask = __ballot_sync(FULL, alive);
             }
+            if constexpr (FINAL) {
+                if (lane < ne) Env::store_trace(st, final_row(p, id, e0 + lane, Env::STATE_DIM));
+            }
             if constexpr (EVAL) {
                 if (lane < ne) {
                     const size_t at = (size_t)(id / p.layout.group) * p.eval_episodes + m0 + lane;
@@ -288,7 +292,8 @@ static int launch_rollout_gru_generic(int num_sms, int ctas_per_sm, const Rollou
     constexpr int EC = GruGenConfig<Env>::EC, WARPS = GruGenConfig<Env>::WARPS;
     const size_t smem = WARPS * sizeof(GruGenSmem<Env, EC>);
     auto kern = EVAL ? (trace ? k_rollout_gru_generic<Env, EC, WARPS, true, true> : k_rollout_gru_generic<Env, EC, WARPS, false, true>)
-              : trace ? k_rollout_gru_generic<Env, EC, WARPS, true> : k_rollout_gru_generic<Env, EC, WARPS, false>;
+              : trace ? k_rollout_gru_generic<Env, EC, WARPS, true>
+              : rp.final_states ? k_rollout_gru_generic<Env, EC, WARPS, false, false, true> : k_rollout_gru_generic<Env, EC, WARPS, false>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     int per_sm = 0;
     if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, WARPS * 32, smem);

@@ -99,7 +99,16 @@ struct RolloutParams {
     // [n_pol][eval_episodes][max_step][state_dim | n_agents] and eval_returns is unused
     double *trace_returns;       // [n_pol][eval_episodes][max_step] return after each step
     double *trace_initial;       // [eval_episodes][state_dim] initial states (layout of init_states rows), written by policy 0
+    // final states (the FINAL instances, ses_set_final_states): the state after each training episode's last step, in the
+    // layout of Env::store_trace, at row (global id) * E + episode of [P][E][state_dim]; only the ids this handle owns
+    double *final_states;
 };
+
+// row of (offspring id, episode e) in the final-state buffer: 64-bit, P * E * state_dim passes 2^31
+__device__ __forceinline__ double *final_row(const RolloutParams &p, int id, int e, int state_dim)
+{
+    return p.final_states + ((size_t)id * p.E + e) * state_dim;
+}
 
 // row of (episode m of policy j, step t) in the recording buffers: 64-bit, n_pol * eval_episodes * max_step * state_dim
 // passes 2^31 quickly
@@ -217,9 +226,10 @@ template <class Env> struct EnvSplit<Env, decltype((void)Env::SPLIT)> { static c
 // episodes are compacted -- episode g moves to lanes [K g, K g + K) with its state replicated -- and stepped by K lanes each
 // until they end, or until so few are left that twice as many lanes per episode fit (K = 2 -> 4).  A finished episode is
 // booked into its slot (steps, ep_done) exactly as the throughput loop does; the caller retires the slots afterwards.
-template <class Env, int S, int K, class Smem>
+template <class Env, int S, int K, bool FINAL = false, class Smem>
 __device__ __forceinline__ void run_split(Smem &sm, int pomdp, int max_step, int lane, bool &active, int &slot, int &nstep, double &x,
-                                          double &xd, double &th, double &thd)
+                                          double &xd, double &th, double &thd, [[maybe_unused]] int *ep = nullptr,
+                                          [[maybe_unused]] double *final_states = nullptr, [[maybe_unused]] int E = 0)
 {
     static_assert(Env::UNIT_REWARD && Env::N_AGENTS == 1, "run_split: CartPole-like envs");
     const unsigned FULL = 0xffffffffu;
@@ -230,6 +240,7 @@ __device__ __forceinline__ void run_split(Smem &sm, int pomdp, int max_step, int
     x = __shfl_sync(FULL, x, src); xd = __shfl_sync(FULL, xd, src);
     th = __shfl_sync(FULL, th, src); thd = __shfl_sync(FULL, thd, src);
     slot = __shfl_sync(FULL, slot, src); nstep = __shfl_sync(FULL, nstep, src);
+    if constexpr (FINAL) *ep = __shfl_sync(FULL, *ep, src);
     active = g < n_act;
     if (!active) slot = 0;                                                // idle groups step a dummy episode (result unused)
     typename Env::template SplitW<K> wr;
@@ -245,6 +256,10 @@ __device__ __forceinline__ void run_split(Smem &sm, int pomdp, int max_step, int
             if (nstep >= max_step) done = true;
             if (done) {
                 if ((lane & (K - 1)) == 0) {
+                    if constexpr (FINAL) {
+                        double *row = final_states + ((size_t)sm.off_id[slot] * E + *ep) * 4;
+                        row[0] = x; row[1] = xd; row[2] = th; row[3] = thd;
+                    }
                     atomicAdd(&sm.steps[slot], nstep);
                     atomicAdd(&sm.ep_done[slot], 1);
                 }
@@ -272,11 +287,28 @@ __device__ __noinline__ void split_phase(Smem *smp, int pomdp, int max_step, int
         run_split<Env, S, 4>(sm, pomdp, max_step, lane, active, slot, nstep, x, xd, th, thd);      // runs them to their end
 }
 
+// The straggler phase of the FINAL instances: as split_phase, and the lane that ends an episode stores its final state.  A
+// function of its own so that split_phase keeps its signature and code.
+template <class Env, int S, class Smem>
+__device__ __noinline__ void split_phase_final(Smem *smp, int pomdp, int max_step, int slot, int nstep, double x, double xd, double th,
+                                               double thd, int ep, double *final_states, int E)
+{
+    Smem &sm = *smp;
+    const int lane = threadIdx.x & 31;
+    bool active = slot >= 0;
+    if (__popc(__ballot_sync(0xffffffffu, active)) > 8)
+        run_split<Env, S, 2, true>(sm, pomdp, max_step, lane, active, slot, nstep, x, xd, th, thd, &ep, final_states, E);
+    if (__ballot_sync(0xffffffffu, active))
+        run_split<Env, S, 4, true>(sm, pomdp, max_step, lane, active, slot, nstep, x, xd, th, thd, &ep, final_states, E);
+}
+
 // PEER: the instance launched when the launch ends with the peer flag barrier (sentinel CTA + one atomic at the workers' end); a
 // separate instance so that single-GPU launches keep the exact code they have without it.
 // EVAL: the policy-evaluation instance (ses_evaluate): unperturbed policies, STREAM_EVAL initial states, per-episode returns and
 // lengths instead of fitness; no straggler phase.  Separate so that the training instances keep their code.
-template <class Env, int S, int WARPS, bool TRACE, bool PEER = false, bool EVAL = false>
+// FINAL: the training instance that also stores the final state of every episode (p.final_states), written by the lane that
+// ends the episode, in the throughput loop or the straggler phase.  Separate for the same reason.
+template <class Env, int S, int WARPS, bool TRACE, bool PEER = false, bool EVAL = false, bool FINAL = false>
 __global__ void __launch_bounds__(WARPS * 32) k_rollout_slots(const RolloutParams p)
 {
     using Smem = SlotSmem<Env, S, !Env::UNIT_REWARD>;
@@ -513,6 +545,7 @@ __global__ void __launch_bounds__(WARPS * 32) k_rollout_slots(const RolloutParam
                 } else if constexpr (!Env::UNIT_REWARD) {
                     sm.ret[slot][ep] = st.ret;
                 }
+                if constexpr (FINAL) Env::store_trace(st, final_row(p, sm.off_id[slot], ep, Env::STATE_DIM));
                 atomicAdd(&sm.steps[slot], nstep);
                 atomicAdd(&sm.ep_done[slot], 1);
                 slot = -1;
@@ -527,7 +560,8 @@ __global__ void __launch_bounds__(WARPS * 32) k_rollout_slots(const RolloutParam
         // ------------------------------------------------------------------ straggler phase (kept out of the loop above so
         // that its code does not touch the throughput loop's register allocation and schedule)
         if (to_split) {
-            split_phase<Env, S, Smem>(&sm, p.pomdp, p.max_step, slot, nstep, st.x, st.xd, st.th, st.thd);
+            if constexpr (FINAL) split_phase_final<Env, S, Smem>(&sm, p.pomdp, p.max_step, slot, nstep, st.x, st.xd, st.th, st.thd, ep, p.final_states, p.E);
+            else split_phase<Env, S, Smem>(&sm, p.pomdp, p.max_step, slot, nstep, st.x, st.xd, st.th, st.thd);
             __syncwarp();
             if (lane < S && sm.off_id[lane] >= 0) retire_slot<Env>(sm, p, lane, warp_steps);   // every slot the warp still holds
         }

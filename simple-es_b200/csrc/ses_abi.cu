@@ -14,6 +14,7 @@
 #include <cstdlib>
 #include <cstring>
 
+#include "novelty.cuh"
 #include "rank.cuh"
 #include "rollout_cartpole_mlp.cuh"
 #include "rollout_cartpole_gru.cuh"
@@ -102,6 +103,7 @@ struct ses_handle {
     bool peer_fold = false;                       // test build, SES_PEER_FOLD=1: the barriers run inside K1 / k_grad_partial (PeerSync)
     bool barrier_folded = false;                  // that rollout's launch ended with the flag barrier: the next ses_peer_barrier() is a no-op
     unsigned long long *step_counter = nullptr;   // caller-owned, optional (ses_set_step_counter)
+    double *final_states = nullptr;               // caller-owned, optional [P][E][state_dim] (ses_set_final_states)
     // rollout launch configuration
     int lanes_used_override = 0;
     int ctas_per_sm = 0;
@@ -256,6 +258,13 @@ extern "C" int ses_set_step_counter(ses_handle *h, uint64_t *counter_dev)
     return 0;
 }
 
+extern "C" int ses_set_final_states(ses_handle *h, double *final_states_dev)
+{
+    if (!h) return fail("ses_set_final_states: null handle");
+    h->final_states = final_states_dev;
+    return 0;
+}
+
 // ------------------------------------------------------------------------------------------------
 // K1
 // ------------------------------------------------------------------------------------------------
@@ -268,12 +277,13 @@ static int launch_slots(ses_handle *h, RolloutParams &rp, int need_warps, bool t
 #ifdef SES_BUILD_TESTS
     // SES_PEER_FOLD=1 (test build): the launch ends with the peer flag barrier (PeerSync, sentinel CTA).  Measured and not
     // adopted: two launches fewer per generation but 0.782 instead of 0.772 ms at N = 8 (profiles/r02_k1_experiments.md section 11)
-    const bool fold = rp.n_peers > 0 && h->peer_fold && !trace;
+    const bool fold = rp.n_peers > 0 && h->peer_fold && !trace && !rp.final_states;
     auto kernel = trace ? k_rollout_slots<Env, SL, WARPS, true> : fold ? k_rollout_slots<Env, SL, WARPS, false, true> : k_rollout_slots<Env, SL, WARPS, false>;
 #else
     [[maybe_unused]] const bool fold = false;
     auto kernel = trace ? k_rollout_slots<Env, SL, WARPS, true> : k_rollout_slots<Env, SL, WARPS, false>;
 #endif
+    if (rp.final_states) kernel = k_rollout_slots<Env, SL, WARPS, false, false, false, true>;   // the final-state instance
     const size_t smem = WARPS * sizeof(Smem);
     rp.slots_cap = SL;
     CU(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -382,6 +392,7 @@ extern "C" int ses_rollout(ses_handle *h, uint32_t generation, float sigma, cons
     if (!fitness_dev || !steps_dev) return fail("ses_rollout: fitness_dev and steps_dev are required");
     if (!parents_dev && !w_override_dev) return fail("ses_rollout: need parents_dev or w_override_dev");
     if (n_trace > 0 && (!trace_dev || !trace_actions_dev)) return fail("ses_rollout: n_trace > 0 needs trace buffers");
+    if (n_trace > 0 && h->final_states) return fail("ses_rollout: traces and final states (ses_set_final_states) cannot be stored in one launch");
     const ses_config &c = h->cfg;
     const int n_local = h->shard.n_local;
     if (n_local == 0) return 0;
@@ -411,6 +422,7 @@ extern "C" int ses_rollout(ses_handle *h, uint32_t generation, float sigma, cons
         h->last_rollout_fitness = rp.n_peers > 0 ? fitness_dev : nullptr;
     }
     rp.sync.world = 0;
+    rp.final_states = h->final_states;
     h->barrier_folded = false;
 
     // lanes per warp and the grid are chosen per kernel in launch_slots(); the GRU kernel maps a warp to one offspring
@@ -569,6 +581,69 @@ extern "C" int ses_record(ses_handle *h, uint32_t round, const float *policies_d
     rp.trace_initial = initial_dev; rp.trace = states_dev; rp.trace_actions = actions_dev; rp.trace_returns = returns_dev;
     rp.eval_lengths = lengths_dev;
     return launch_eval(h, "ses_record", round, policies_dev, n_pol, n_episodes, init_states_dev, rp, true, stream);
+}
+
+// ------------------------------------------------------------------------------------------------
+// novelty search (DESIGN.md section 4.10): behaviour characterisations, archive novelty, blended shaping
+// ------------------------------------------------------------------------------------------------
+extern "C" int ses_behavior(ses_handle *h, const double *final_states_dev, int32_t n, double *bc_dev, void *stream)
+{
+    if (!h) return fail("ses_behavior: null handle");
+    if (!final_states_dev || !bc_dev) return fail("ses_behavior: final_states_dev and bc_dev are required");
+    if (n < 1 || n > h->cfg.population) return fail("ses_behavior: n=%d outside [1, population=%d]", n, h->cfg.population);
+    CU(cudaSetDevice(h->cfg.device));
+    const long long total = (long long)n * h->state_dim;
+    k_behavior<<<(unsigned)((total + 255) / 256), 256, 0, S(stream)>>>(final_states_dev, n, h->cfg.eval_ep_num, h->state_dim, bc_dev);
+    CU(cudaGetLastError());
+    h->launches += 1;
+    return 0;
+}
+
+template <int SD>
+static void launch_novelty(const double *bc, int n, const double *archive, int n_archive, int k, double *novelty, cudaStream_t st)
+{
+    const int grid = (n + NOVELTY_THREADS - 1) / NOVELTY_THREADS;
+    if (k <= 1) k_novelty<SD, 1><<<grid, NOVELTY_THREADS, 0, st>>>(bc, n, archive, n_archive, k, novelty);
+    else if (k <= 2) k_novelty<SD, 2><<<grid, NOVELTY_THREADS, 0, st>>>(bc, n, archive, n_archive, k, novelty);
+    else if (k <= 4) k_novelty<SD, 4><<<grid, NOVELTY_THREADS, 0, st>>>(bc, n, archive, n_archive, k, novelty);
+    else if (k <= 8) k_novelty<SD, 8><<<grid, NOVELTY_THREADS, 0, st>>>(bc, n, archive, n_archive, k, novelty);
+    else if (k <= 16) k_novelty<SD, 16><<<grid, NOVELTY_THREADS, 0, st>>>(bc, n, archive, n_archive, k, novelty);
+    else k_novelty<SD, 32><<<grid, NOVELTY_THREADS, 0, st>>>(bc, n, archive, n_archive, k, novelty);
+}
+
+extern "C" int ses_novelty(ses_handle *h, const double *bc_dev, int32_t n, const double *archive_dev, int32_t n_archive, int32_t k,
+                           double *novelty_dev, void *stream)
+{
+    if (!h) return fail("ses_novelty: null handle");
+    if (!bc_dev || !archive_dev || !novelty_dev) return fail("ses_novelty: bc_dev, archive_dev and novelty_dev are required");
+    if (n < 1 || n > h->cfg.population) return fail("ses_novelty: n=%d outside [1, population=%d]", n, h->cfg.population);
+    if (n_archive < 1) return fail("ses_novelty: n_archive must be >= 1 (got %d)", n_archive);
+    if (k < 1 || k > NOVELTY_MAX_K) return fail("ses_novelty: k must be in [1, %d] (got %d)", NOVELTY_MAX_K, k);
+    CU(cudaSetDevice(h->cfg.device));
+    switch (h->state_dim) {                     // MountainCar / Pendulum, CartPole / Acrobot, simple_spread N = 2, N = 3
+    case 2: launch_novelty<2>(bc_dev, n, archive_dev, n_archive, k, novelty_dev, S(stream)); break;
+    case 4: launch_novelty<4>(bc_dev, n, archive_dev, n_archive, k, novelty_dev, S(stream)); break;
+    case 8: launch_novelty<8>(bc_dev, n, archive_dev, n_archive, k, novelty_dev, S(stream)); break;
+    case 12: launch_novelty<12>(bc_dev, n, archive_dev, n_archive, k, novelty_dev, S(stream)); break;
+    default: return fail("ses_novelty: no kernel for state_dim %d", h->state_dim);
+    }
+    CU(cudaGetLastError());
+    h->launches += 1;
+    return 0;
+}
+
+extern "C" int ses_blend_shaped(ses_handle *h, const double *shaped_f_dev, const double *shaped_n_dev, int32_t n, double w,
+                                double *out_dev, void *stream)
+{
+    if (!h) return fail("ses_blend_shaped: null handle");
+    if (!shaped_f_dev || !shaped_n_dev || !out_dev) return fail("ses_blend_shaped: shaped_f_dev, shaped_n_dev and out_dev are required");
+    if (n < 1 || n > h->cfg.population) return fail("ses_blend_shaped: n=%d outside [1, population=%d]", n, h->cfg.population);
+    if (!(w >= 0.0 && w <= 1.0)) return fail("ses_blend_shaped: w must be in [0, 1] (got %g)", w);
+    CU(cudaSetDevice(h->cfg.device));
+    k_blend_shaped<<<(n + 255) / 256, 256, 0, S(stream)>>>(shaped_f_dev, shaped_n_dev, n, w, out_dev);
+    CU(cudaGetLastError());
+    h->launches += 1;
+    return 0;
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -32,14 +32,14 @@ def init_from_env(backend=None):
 
 
 def exchange_fitness(fitness, lo, hi):
-    """Make the full fitness vector [P] available on every rank; `fitness[lo:hi]` holds this rank's
-    slice on entry.  Equal shards: one all_gather (NCCL over NVLink).  Ragged shards
+    """Make the full fitness vector [P] (or any [P, ...] tensor, e.g. nsr_es's final states) available on every rank;
+    `fitness[lo:hi]` holds this rank's slice on entry.  Equal shards: one all_gather (NCCL over NVLink).  Ragged shards
     (simple_evolution's P = n + 1): all_reduce(SUM) of the zero-padded vector, which is exact
     because x + 0.0 == x."""
     rank, ws = world()
     if ws == 1:
         return fitness
-    P = fitness.numel()
+    P = fitness.shape[0]
     if P % ws == 0:
         dist.all_gather_into_tensor(fitness, fitness[lo:hi].clone())
     else:
@@ -50,12 +50,12 @@ def exchange_fitness(fitness, lo, hi):
 
 
 def exchange_fitness_masked(fitness, not_mine):
-    """The same for a non-contiguous (block-cyclic) slice: `not_mine` is a bool mask of the entries other ranks own.
-    all_reduce(SUM) of the vector with those entries zeroed -- exact, every entry has exactly one non-zero contributor."""
+    """The same for a non-contiguous (block-cyclic) slice: `not_mine` is a bool mask [P] of the rows other ranks own.
+    all_reduce(SUM) of the tensor with those rows zeroed -- exact, every entry has exactly one non-zero contributor."""
     rank, ws = world()
     if ws == 1:
         return fitness
-    fitness.masked_fill_(not_mine, 0.0)
+    fitness.masked_fill_(not_mine.view((-1,) + (1,) * (fitness.dim() - 1)), 0.0)
     dist.all_reduce(fitness, op=dist.ReduceOp.SUM)
     return fitness
 

@@ -36,7 +36,7 @@ def population_layout(strategy, offspring_num, elite_num=None):
     n = int(offspring_num)
     if strategy == "simple_evolution":
         return n + 1, n + 1, 2, 1            # [mu, elite0 (== mu), n-1 perturbed]
-    if strategy == "openai_es":
+    if strategy in ("openai_es", "nsr_es"):
         return n, n, 1, 1                    # [mu, n-1 perturbed]
     if strategy == "simple_genetic":
         k = int(elite_num)
@@ -184,6 +184,55 @@ class RolloutEngine:
         self._chk(counter, torch.int64, 1, "counter")
         self._step_counter = counter            # keep alive
         self._check(self.lib.ses_set_step_counter(self._h, _ptr(counter)))
+
+    def set_final_states(self, final_states):
+        """`final_states`: [P, E, state_dim] float64 CUDA tensor, or None (off).  While set, every rollout() also stores the
+        state after each episode's last step in the rows of the ids this engine owns (DESIGN.md section 4.10)."""
+        self._chk(final_states, torch.float64, self.P * self.E * self.state_dim, "final_states")
+        self._final_states = final_states       # keep alive
+        self._check(self.lib.ses_set_final_states(self._h, _ptr(final_states)))
+
+    # ------------------------------------------------------------------------------ novelty search (nsr_es)
+    def behavior(self, final_states, out=None):
+        """Behaviour characterisations [n, state_dim] f64: the mean over episodes of final_states [n, E, state_dim]."""
+        self._chk(final_states, torch.float64, name="final_states")
+        n = final_states.numel() // (self.E * self.state_dim)
+        if final_states.numel() != n * self.E * self.state_dim:
+            raise ValueError("final_states has %d elements, not a multiple of E * state_dim = %d"
+                             % (final_states.numel(), self.E * self.state_dim))
+        if out is None:
+            out = torch.empty((n, self.state_dim), dtype=torch.float64, device=self.device)
+        self._chk(out, torch.float64, n * self.state_dim, "out")
+        self._check(self.lib.ses_behavior(self._h, _ptr(final_states), n, _ptr(out), self._stream()))
+        return out
+
+    def novelty(self, bc, archive, n_archive, k, out=None):
+        """novelty [n] f64: mean distance from each row of bc [n, state_dim] to its min(k, n_archive) nearest rows of
+        archive[:n_archive] (archive: [>= n_archive, state_dim] f64)."""
+        self._chk(bc, torch.float64, name="bc")
+        self._chk(archive, torch.float64, name="archive")
+        n = bc.numel() // self.state_dim
+        if bc.numel() != n * self.state_dim:
+            raise ValueError("bc has %d elements, not a multiple of state_dim = %d" % (bc.numel(), self.state_dim))
+        if archive.numel() < int(n_archive) * self.state_dim:
+            raise ValueError("archive has %d elements, fewer than n_archive * state_dim = %d"
+                             % (archive.numel(), int(n_archive) * self.state_dim))
+        if out is None:
+            out = torch.empty(n, dtype=torch.float64, device=self.device)
+        self._chk(out, torch.float64, n, "out")
+        self._check(self.lib.ses_novelty(self._h, _ptr(bc), n, _ptr(archive), int(n_archive), int(k), _ptr(out), self._stream()))
+        return out
+
+    def blend_shaped(self, shaped_f, shaped_n, w, out=None):
+        """(1 - w) shaped_f + w shaped_n, float64, each operation separately rounded."""
+        self._chk(shaped_f, torch.float64, name="shaped_f")
+        n = shaped_f.numel()
+        self._chk(shaped_n, torch.float64, n, "shaped_n")
+        if out is None:
+            out = torch.empty(n, dtype=torch.float64, device=self.device)
+        self._chk(out, torch.float64, n, "out")
+        self._check(self.lib.ses_blend_shaped(self._h, _ptr(shaped_f), _ptr(shaped_n), n, float(w), _ptr(out), self._stream()))
+        return out
 
     # ------------------------------------------------------------------------------ K1
     def rollout(self, generation, sigma, parents, fitness=None, steps=None, w_override=None, init_states=None,

@@ -1,4 +1,5 @@
-"""Device-resident strategy state for the three offspring strategies.
+"""Device-resident strategy state for the offspring strategies: the reference's three, and nsr_es (novelty search with
+reward), an opt-in addition.
 
 Each class keeps what the reference strategy keeps (learning_strategies/evolution/offspring_strategies.py)
 -- mu / elite table, sigma, Adam moments -- as a few small CUDA tensors, and never materialises the
@@ -193,9 +194,13 @@ class OpenAIES(_Base):
         self.momentum = float(self.engine_cfg.get("momentum", 0.9))
 
     def step(self):
-        e = self.engine
         self._rollout_and_exchange()
-        e.rank_desc(self.fitness, shaped=True, order=self.order, shaped_out=self.shaped)
+        self.engine.rank_desc(self.fitness, shaped=True, order=self.order, shaped_out=self.shaped)
+        self._update()
+
+    def _update(self):
+        """K3 from self.shaped, then the sigma decay and the next generation."""
+        e = self.engine
         self.t += 1
         if self.optimizer == "sgd":
             e.update_openai_sgd(self.generation, self.sigma, self.lr, self.shaped, self.parents.view(-1), self.v, self.momentum)
@@ -248,4 +253,86 @@ class SimpleGenetic(_Base):
         return self.parents[0]                                    # elite_models[0] (:64-65)
 
 
-STRATEGIES = {c.name: c for c in (OpenAIES, SimpleEvolution, SimpleGenetic)}
+def _novelty_params(cfg):
+    """(novelty_weight, novelty_k) of an nsr_es strategy section, validated."""
+    allowed = {"name", "init_sigma", "sigma_decay", "learning_rate", "offspring_num", "novelty_weight", "novelty_k"}
+    unknown = sorted(set(cfg) - allowed)
+    if unknown:
+        raise ValueError("strategy nsr_es: unknown key(s) %s (allowed: %s)" % (", ".join(unknown), ", ".join(sorted(allowed))))
+    w, k = cfg.get("novelty_weight", 0.5), cfg.get("novelty_k", 10)
+    if isinstance(w, bool) or not isinstance(w, (int, float)) or not 0.0 <= float(w) <= 1.0:
+        raise ValueError("strategy nsr_es: novelty_weight must be a number in [0, 1] (got %r)" % (w,))
+    if isinstance(k, bool) or not isinstance(k, int) or not 1 <= k <= 32:
+        raise ValueError("strategy nsr_es: novelty_k must be an integer in [1, 32] (got %r)" % (k,))
+    return float(w), int(k)
+
+
+class NoveltyES(OpenAIES):
+    """openai_es plus novelty (NSR-ES, Conti et al. 2018; opt-in, the reference has no such strategy).  The same population,
+    update and sigma decay as openai_es, but K3 follows (1 - w) * the centered ranks of fitness + w * the centered ranks of
+    novelty.  An offspring's behaviour is the mean of its episodes' final states; its novelty is the mean distance to the k
+    nearest behaviours in the archive, which holds mu's behaviour of every generation so far (DESIGN.md section 4.10).
+    w = 0 trains exactly as openai_es."""
+    name = "nsr_es"
+
+    def __init__(self, strategy_cfg, *a, **kw):
+        self.novelty_weight, self.novelty_k = _novelty_params(strategy_cfg)
+        super().__init__(strategy_cfg, *a, **kw)
+        e, dev = self.engine, self.engine.device
+        self._run_key.update(novelty_k=self.novelty_k, novelty_weight=self.novelty_weight)
+        self.final_states = torch.zeros((self.P, e.E, e.state_dim), dtype=torch.float64, device=dev)
+        e.set_final_states(self.final_states)
+        self.bc = torch.empty((self.P, e.state_dim), dtype=torch.float64, device=dev)
+        self.novelty = torch.empty(self.P, dtype=torch.float64, device=dev)
+        self.novelty_order = torch.empty(self.P, dtype=torch.int32, device=dev)
+        self.shaped_f = torch.empty(self.P, dtype=torch.float64, device=dev)
+        self.shaped_n = torch.empty(self.P, dtype=torch.float64, device=dev)
+        self.archive = torch.empty((16, e.state_dim), dtype=torch.float64, device=dev)   # grows by doubling
+        self.n_archive = 0
+        if self.shard and not hasattr(self, "_not_mine"):
+            mask = torch.ones(self.P, dtype=torch.bool)
+            mask[torch.from_numpy(owned_ids(self.P, *self.shard))] = False
+            self._not_mine = mask.to(dev)
+
+    def _reserve(self, n):
+        if n > self.archive.shape[0]:
+            grown = torch.empty((max(16, 1 << (n - 1).bit_length()), self.archive.shape[1]), dtype=torch.float64,
+                                device=self.archive.device)
+            grown[:self.n_archive].copy_(self.archive[:self.n_archive])
+            self.archive = grown
+
+    def step(self):
+        e = self.engine
+        self._rollout_and_exchange()                   # K1 also stores every episode's final state (set_final_states)
+        if sdist.world()[1] > 1:                       # every rank gets every row, exactly; then all compute the same
+            if self.shard:
+                sdist.exchange_fitness_masked(self.final_states, self._not_mine)
+            else:
+                sdist.exchange_fitness(self.final_states, self.lo, self.hi)
+        e.behavior(self.final_states, out=self.bc)
+        self._reserve(self.n_archive + 1)
+        self.archive[self.n_archive].copy_(self.bc[0])   # mu's behaviour joins the archive before novelty is measured
+        self.n_archive += 1
+        e.novelty(self.bc, self.archive, self.n_archive, self.novelty_k, out=self.novelty)
+        e.rank_desc(self.fitness, shaped=True, order=self.order, shaped_out=self.shaped_f)
+        e.rank_desc(self.novelty, shaped=True, order=self.novelty_order, shaped_out=self.shaped_n, full_key=True)
+        e.blend_shaped(self.shaped_f, self.shaped_n, self.novelty_weight, out=self.shaped)
+        self._update()
+
+    def state(self):
+        st = super().state()
+        st["archive"] = self.archive[:self.n_archive].detach().cpu().clone()
+        return st
+
+    def load_state(self, st):
+        super().load_state(st)
+        a = st["archive"]
+        if a.dim() != 2 or a.shape[1] != self.archive.shape[1]:
+            raise ValueError("resume state has an archive of shape %s, this run needs [n, %d]" % (tuple(a.shape), self.archive.shape[1]))
+        self.n_archive = 0
+        self._reserve(a.shape[0])
+        self.archive[:a.shape[0]].copy_(a)
+        self.n_archive = int(a.shape[0])
+
+
+STRATEGIES = {c.name: c for c in (OpenAIES, SimpleEvolution, SimpleGenetic, NoveltyES)}
