@@ -281,6 +281,10 @@ TW_EXPORT void tw_classic_init(int env, uint32_t seed, int init_mode, uint32_t g
 TW_EXPORT double tw_rollout_classic_gru(int env, int gru, const float *w, int E, int max_step, const double *init, uint32_t seed,
                                         int init_mode, uint32_t gen, uint32_t id, double *trace, int32_t *actions,
                                         int trace_steps, int64_t *steps_out);
+/* final: optional [E][state_dim] state after each episode's last step. */
+static double classic_rollout(int env, int gru, const float *w, int E, int max_step, const double *init, uint32_t seed,
+                              int init_mode, uint32_t gen, uint32_t id, double *trace, int32_t *actions, int trace_steps,
+                              int64_t *steps_out, double *final);
 
 /* One offspring: E episodes (loop.py:111-125).  Returns fitness = (sum over episodes, in episode order, of the
  * sequential float64 sum of the episode's rewards) / E.
@@ -298,6 +302,13 @@ TW_EXPORT double tw_rollout_classic(int env, const float *w, int E, int max_step
 TW_EXPORT double tw_rollout_classic_gru(int env, int gru, const float *w, int E, int max_step, const double *init, uint32_t seed,
                                         int init_mode, uint32_t gen, uint32_t id, double *trace, int32_t *actions,
                                         int trace_steps, int64_t *steps_out)
+{
+    return classic_rollout(env, gru, w, E, max_step, init, seed, init_mode, gen, id, trace, actions, trace_steps, steps_out, NULL);
+}
+
+static double classic_rollout(int env, int gru, const float *w, int E, int max_step, const double *init, uint32_t seed,
+                              int init_mode, uint32_t gen, uint32_t id, double *trace, int32_t *actions, int trace_steps,
+                              int64_t *steps_out, double *final)
 {
     int obs, act, sd, cap;
     if (tw_classic_dims(env, &obs, &act, &sd, &cap)) return NAN;
@@ -333,6 +344,7 @@ TW_EXPORT double tw_rollout_classic_gru(int env, int gru, const float *w, int E,
                 if (actions) actions[step - 1] = a;
             }
         }
+        if (final) memcpy(final + (size_t)sd * e, st, sizeof(double) * (size_t)sd);
         nsteps += step;
         total = total + R;
     }
@@ -344,7 +356,8 @@ typedef struct {
     int env; const float *parents; float sigma; uint32_t seed, gen; int group, n_head, id0, n, E, max_step;
     const float *W_override; const double *init; int init_mode; double *fitness; int64_t *steps; int D;
     atomic_int next;
-    int gru;
+    int gru, sd;
+    double *final;
 } classic_job;
 
 static void *classic_worker(void *arg)
@@ -359,8 +372,9 @@ static void *classic_worker(void *arg)
             if (jb->W_override) memcpy(w, jb->W_override + (size_t)j * jb->D, sizeof(float) * (size_t)jb->D);
             else tw_perturb(jb->parents + (size_t)(id / jb->group) * jb->D, jb->D, jb->sigma, jb->seed, jb->gen, (uint32_t)id,
                             (id % jb->group) - jb->n_head + 1, w);
-            jb->fitness[j] = tw_rollout_classic_gru(jb->env, jb->gru, w, jb->E, jb->max_step, jb->init, jb->seed, jb->init_mode, jb->gen,
-                                                    (uint32_t)id, NULL, NULL, 0, &jb->steps[j]);
+            jb->fitness[j] = classic_rollout(jb->env, jb->gru, w, jb->E, jb->max_step, jb->init, jb->seed, jb->init_mode, jb->gen,
+                                             (uint32_t)id, NULL, NULL, 0, &jb->steps[j],
+                                             jb->final ? jb->final + (size_t)j * jb->E * jb->sd : NULL);
         }
     }
     free(w);
@@ -369,12 +383,13 @@ static void *classic_worker(void *arg)
 
 TW_EXPORT void tw_population_classic_gru(int env, int gru, const float *parents, float sigma, uint32_t seed, uint32_t gen, int group,
                                          int n_head, int id0, int n, int E, int max_step, const float *W_override,
-                                         const double *init, int init_mode, double *fitness, int64_t *steps, int nthreads)
+                                         const double *init, int init_mode, double *fitness, int64_t *steps, int nthreads,
+                                         double *final)
 {
     int obs, act, sd, cap;
     if (tw_classic_dims(env, &obs, &act, &sd, &cap)) return;
     classic_job jb = { env, parents, sigma, seed, gen, group, n_head, id0, n, E, max_step, W_override, init, init_mode,
-                       fitness, steps, tw_param_count(obs, act, gru), 0, gru };
+                       fitness, steps, tw_param_count(obs, act, gru), 0, gru, sd, final };
     if (nthreads < 1) nthreads = 1;
     if (nthreads > 256) nthreads = 256;
     pthread_t th[256];
@@ -388,5 +403,5 @@ TW_EXPORT void tw_population_classic(int env, const float *parents, float sigma,
                                      const double *init, int init_mode, double *fitness, int64_t *steps, int nthreads)
 {
     tw_population_classic_gru(env, 0, parents, sigma, seed, gen, group, n_head, id0, n, E, max_step, W_override, init, init_mode,
-                              fitness, steps, nthreads);
+                              fitness, steps, nthreads, NULL);
 }

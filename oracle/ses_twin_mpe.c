@@ -219,6 +219,9 @@ TW_EXPORT void tw_spread_init(uint32_t seed, int init_mode, uint32_t gen, uint32
 TW_EXPORT double tw_rollout_mpe_gru(int gru, const float *w, int N, int E, int max_cycles, const double *init, uint32_t seed,
                                     int init_mode, uint32_t gen, uint32_t id, double *trace, int32_t *actions, int trace_steps,
                                     int64_t *steps_out);
+static double mpe_rollout(int gru, const float *w, int N, int E, int max_cycles, const double *init, uint32_t seed, int init_mode,
+                          uint32_t gen, uint32_t id, double *trace, int32_t *actions, int trace_steps, int64_t *steps_out,
+                          double *final);
 
 TW_EXPORT double tw_rollout_mpe(const float *w, int N, int E, int max_cycles, const double *init, uint32_t seed,
                                 int init_mode, uint32_t gen, uint32_t id, double *trace, int32_t *actions, int trace_steps,
@@ -232,6 +235,14 @@ TW_EXPORT double tw_rollout_mpe(const float *w, int N, int E, int max_cycles, co
 TW_EXPORT double tw_rollout_mpe_gru(int gru, const float *w, int N, int E, int max_cycles, const double *init, uint32_t seed,
                                     int init_mode, uint32_t gen, uint32_t id, double *trace, int32_t *actions, int trace_steps,
                                     int64_t *steps_out)
+{
+    return mpe_rollout(gru, w, N, E, max_cycles, init, seed, init_mode, gen, id, trace, actions, trace_steps, steps_out, NULL);
+}
+
+/* final: optional [E][4N] (agent pos, agent vel) after each episode's last step, laid out as a trace row. */
+static double mpe_rollout(int gru, const float *w, int N, int E, int max_cycles, const double *init, uint32_t seed, int init_mode,
+                          uint32_t gen, uint32_t id, double *trace, int32_t *actions, int trace_steps, int64_t *steps_out,
+                          double *final)
 {
     const int obs = 6 * N;
     double total = 0.0;
@@ -266,6 +277,11 @@ TW_EXPORT double tw_rollout_mpe_gru(int gru, const float *w, int N, int E, int m
                 if (actions) for (int i = 0; i < N; ++i) actions[(size_t)t * N + i] = act[i];
             }
         }
+        if (final) for (int i = 0; i < N; ++i) {
+            double *f = final + (size_t)4 * N * e;
+            f[2 * i] = s.apos[i][0]; f[2 * i + 1] = s.apos[i][1];
+            f[2 * N + 2 * i] = s.avel[i][0]; f[2 * N + 2 * i + 1] = s.avel[i][1];
+        }
         total = total + R;
     }
     if (steps_out) *steps_out = nsteps;
@@ -274,7 +290,7 @@ TW_EXPORT double tw_rollout_mpe_gru(int gru, const float *w, int N, int E, int m
 
 TW_EXPORT void tw_population_mpe_gru(int gru, const float *parents, int N, float sigma, uint32_t seed, uint32_t gen, int group, int n_head,
                                      int id0, int n, int E, int max_cycles, const float *W_override, const double *init,
-                                     int init_mode, double *fitness, int64_t *steps)
+                                     int init_mode, double *fitness, int64_t *steps, double *final)
 {
     const int D = tw_param_count(6 * N, 5, gru);
     float *w = (float *)malloc(sizeof(float) * (size_t)D);
@@ -282,7 +298,8 @@ TW_EXPORT void tw_population_mpe_gru(int gru, const float *parents, int N, float
         int id = id0 + j;
         if (W_override) memcpy(w, W_override + (size_t)j * D, sizeof(float) * (size_t)D);
         else tw_perturb(parents + (size_t)(id / group) * D, D, sigma, seed, gen, (uint32_t)id, (id % group) - n_head + 1, w);
-        fitness[j] = tw_rollout_mpe_gru(gru, w, N, E, max_cycles, init, seed, init_mode, gen, (uint32_t)id, NULL, NULL, 0, &steps[j]);
+        fitness[j] = mpe_rollout(gru, w, N, E, max_cycles, init, seed, init_mode, gen, (uint32_t)id, NULL, NULL, 0, &steps[j],
+                                 final ? final + (size_t)j * E * 4 * N : NULL);
     }
     free(w);
 }
@@ -291,7 +308,7 @@ TW_EXPORT void tw_population_mpe(const float *parents, int N, float sigma, uint3
                                  int id0, int n, int E, int max_cycles, const float *W_override, const double *init,
                                  int init_mode, double *fitness, int64_t *steps)
 {
-    tw_population_mpe_gru(0, parents, N, sigma, seed, gen, group, n_head, id0, n, E, max_cycles, W_override, init, init_mode, fitness, steps);
+    tw_population_mpe_gru(0, parents, N, sigma, seed, gen, group, n_head, id0, n, E, max_cycles, W_override, init, init_mode, fitness, steps, NULL);
 }
 
 TW_EXPORT int tw_spread_policy(const float *w, int N, const float *o, float *logits) { return spread_policy(w, 6 * N, o, logits); }

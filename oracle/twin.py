@@ -167,19 +167,25 @@ def rollout_cartpole(w, gru=False, pomdp=False, E=5, max_step=500, init=None, se
     return int(t), trace[:trace_steps], acts[:trace_steps]
 
 
+def _final(on, n, E, sd):
+    return np.full((n, E, sd), np.nan) if on else None
+
+
 def population_cartpole(parents, gru=False, pomdp=False, sigma=0.0, seed=0, gen=0, group=1, n_head=1, id0=0, n=1,
-                        E=5, max_step=500, W_override=None, init=None, init_mode=0, nthreads=1):
-    """Fitness (float64) and total steps (int64) of offspring [id0, id0+n)."""
+                        E=5, max_step=500, W_override=None, init=None, init_mode=0, nthreads=1, final=False):
+    """Fitness (float64) and total steps (int64) of offspring [id0, id0+n); final=True adds their final states
+    [n][E][4] (the state after each episode's last step)."""
     parents = _f32(parents)
     Wo = None if W_override is None else _f32(W_override)
     init_a = None if init is None else _f64(init)
     fit = np.empty(n, dtype=np.float64)
     steps = np.empty(n, dtype=np.int64)
+    fs = _final(final, n, E, 4)
     lib().tw_population_cartpole(_p(parents), C.c_int(int(gru)), C.c_int(int(pomdp)), C.c_float(sigma),
                                  C.c_uint32(seed), C.c_uint32(gen), C.c_int(group), C.c_int(n_head), C.c_int(id0),
                                  C.c_int(n), C.c_int(E), C.c_int(max_step), _p(Wo), _p(init_a), C.c_int(init_mode),
-                                 _p(fit), _p(steps), C.c_int(nthreads))
-    return fit, steps
+                                 _p(fit), _p(steps), C.c_int(nthreads), _p(fs))
+    return (fit, steps, fs) if final else (fit, steps)
 
 
 # ---------------------------------------------------------------------------- K2 / K3
@@ -263,16 +269,18 @@ def rollout_mpe(w, N=2, E=5, max_cycles=25, init=None, seed=0, init_mode=0, gen=
 
 
 def population_mpe(parents, N=2, sigma=0.0, seed=0, gen=0, group=1, n_head=1, id0=0, n=1, E=5, max_cycles=25,
-                   W_override=None, init=None, init_mode=0, gru=False):
+                   W_override=None, init=None, init_mode=0, gru=False, final=False):
+    """final=True adds the final states [n][E][4N] (agent positions, then velocities, as a trace row)."""
     parents = _f32(parents)
     Wo = None if W_override is None else _f32(W_override)
     init_a = None if init is None else _f64(init)
     fit = np.empty(n, dtype=np.float64)
     steps = np.empty(n, dtype=np.int64)
+    fs = _final(final, n, E, 4 * N)
     lib().tw_population_mpe_gru(C.c_int(int(bool(gru))), _p(parents), C.c_int(N), C.c_float(sigma), C.c_uint32(seed), C.c_uint32(gen),
                                 C.c_int(group), C.c_int(n_head), C.c_int(id0), C.c_int(n), C.c_int(E), C.c_int(max_cycles), _p(Wo),
-                                _p(init_a), C.c_int(init_mode), _p(fit), _p(steps))
-    return fit, steps
+                                _p(init_a), C.c_int(init_mode), _p(fit), _p(steps), _p(fs))
+    return (fit, steps, fs) if final else (fit, steps)
 
 
 # ---------------------------------------------------------------------------- classic control (ses_twin_classic.c)
@@ -331,7 +339,8 @@ def rollout_classic(env, w, E=5, max_step=None, init=None, seed=0, init_mode=0, 
 
 
 def population_classic(env, parents, sigma=0.0, seed=0, gen=0, group=1, n_head=1, id0=0, n=1, E=5, max_step=None,
-                       W_override=None, init=None, init_mode=0, nthreads=8, gru=False):
+                       W_override=None, init=None, init_mode=0, nthreads=8, gru=False, final=False):
+    """final=True adds the final states [n][E][state_dim]."""
     obs, act, sd, cap = classic_dims(env)
     max_step = cap if max_step is None else min(int(max_step), cap)
     parents = _f32(parents)
@@ -339,7 +348,8 @@ def population_classic(env, parents, sigma=0.0, seed=0, gen=0, group=1, n_head=1
     init = None if init is None else _f64(init)
     fitness = np.zeros(n)
     steps = np.zeros(n, dtype=np.int64)
+    fs = _final(final, n, E, sd)
     lib().tw_population_classic_gru(CLASSIC_ENVS[env], int(bool(gru)), _p(parents), C.c_float(sigma), C.c_uint32(seed), C.c_uint32(gen),
                                     int(group), int(n_head), int(id0), int(n), int(E), int(max_step), _p(W_override), _p(init),
-                                    int(init_mode), _p(fitness), _p(steps), int(nthreads))
-    return fitness, steps
+                                    int(init_mode), _p(fitness), _p(steps), int(nthreads), _p(fs))
+    return (fitness, steps, fs) if final else (fitness, steps)

@@ -57,13 +57,51 @@ def novelty(bc, archive, k):
     for i in range(bc.shape[0]):
         diff = bc[i][None, :] - archive
         q = np.zeros(archive.shape[0])
-        for d in range(archive.shape[1]):
-            q = q + diff[:, d] * diff[:, d]
+        with np.errstate(over="ignore"):                     # squares past the float64 range are inf, as on the device
+            for d in range(archive.shape[1]):
+                q = q + diff[:, d] * diff[:, d]
         dist = np.sort(np.sqrt(q))[:m]
         s = 0.0
         for x in dist:
             s = s + x
         out[i] = s / float(m)
+    return out
+
+
+def novelty_table(bc, archive, sizes, ks, chunk=1024, threads=1):
+    """{(a, k): novelty of bc against archive[:a] with k neighbours} for every a in sizes and k in ks: `novelty`, vectorised
+    over rows of bc in chunks (on `threads` host threads) and sharing each chunk's distances between the archive prefixes.
+    The same operations in the same order: q accumulated over d in order from +0, the square root, the min(k, a) smallest
+    distances in ascending order, added left to right from +0 and divided by min(k, a)."""
+    from concurrent.futures import ThreadPoolExecutor
+    bc, archive = np.asarray(bc, dtype=np.float64), np.asarray(archive, dtype=np.float64)
+    sizes, ks = [int(a) for a in sizes], [int(k) for k in ks]
+    out = {(a, k): np.empty(bc.shape[0]) for a in sizes for k in ks}
+
+    def part(lo):
+        hi = min(bc.shape[0], lo + chunk)
+        b = bc[lo:hi]
+        q = np.zeros((hi - lo, max(sizes)))
+        with np.errstate(over="ignore"):
+            for d in range(archive.shape[1]):
+                diff = b[:, d:d + 1] - archive[None, :max(sizes), d]
+                q = q + diff * diff
+        dist = np.sqrt(q)
+        for a in sizes:
+            mmax = min(max(ks), a)
+            near = dist[:, :a] if mmax == a else np.partition(dist[:, :a], mmax - 1, axis=1)[:, :mmax]
+            near = np.sort(near, axis=1)
+            s = np.zeros(hi - lo)
+            sums = []
+            for j in range(mmax):
+                s = s + near[:, j]
+                sums.append(s)
+            for k in ks:
+                m = min(k, a)
+                out[a, k][lo:hi] = sums[m - 1] / float(m)
+
+    with ThreadPoolExecutor(max(1, threads)) as ex:
+        list(ex.map(part, range(0, bc.shape[0], chunk)))
     return out
 
 
