@@ -82,8 +82,9 @@ int ses_destroy(ses_handle *h);
  * env wrappers' reset/step (envs/gym_wrapper.py:23-45, envs/pettingzoo_wrapper.py:22-58) and the
  * perturbation half of _gen_offsprings (offspring_strategies.py:53-60,169-176,312-326).
  *   parents_dev      [n_parents][D] f32
- *   w_override_dev   optional [id_end-id_begin][D] f32: explicit offspring weights (verification
- *                    mode: the reference's own perturbed arrays) instead of Philox perturbation
+ *   w_override_dev   optional [n_local][D] f32 in local order: explicit offspring weights instead of Philox perturbation
+ *                    (sigma is then unused): sep_cma_es's samples (ses_cma_sample), or the reference's own perturbed arrays
+ *                    in verification mode
  *   init_states_dev  optional [E][state_dim] f64 explicit initial states (verification mode);
  *                    NULL -> Philox stream per cfg.init_mode
  *   fitness_dev      [P] f64, written at [id_begin, id_end): total reward / eval_ep_num (loop.py:124)
@@ -225,6 +226,35 @@ int ses_novelty(ses_handle *h, const double *bc_dev, int32_t n, const double *ar
                 double *novelty_dev, void *stream);
 int ses_blend_shaped(ses_handle *h, const double *shaped_f_dev, const double *shaped_n_dev, int32_t n, double w, double *out_dev,
                      void *stream);
+
+/* Separable CMA-ES (the sep_cma_es strategy, DESIGN.md section 4.11; Ros & Hansen 2008).  Needs the layout group = population,
+ * n_head = 0, antithetic = 0: every offspring is sampled.  State, all [D] f64 device vectors unless noted: mean m, diagonal
+ * covariance c, evolution paths p_sigma and p_c, and sigma ([1] f64, on the device because it depends on |p_sigma|).  float64
+ * with each operation separately rounded; sigma goes through the device exp (<= 1 ulp), everything else is defined bit for bit.
+ * ses_cma_sample: out_dev [n_local][D] f32, row l = (float)(m + sigma (sqrt(c) z)) for the id this handle holds at local index l
+ *                 (ses_rollout's w_override order), z[d] = the Philox normal of (generation, id) that K3 re-derives.
+ * ses_cma_update: one generation's update from order_dev [population] (ses_rank_desc of the full fitness vector):
+ *                 s_dev [population] f64 := weights_dev[r] at order[r] for r < mu, else 0 (weights_dev [mu] f64);
+ *                 <z> = sum_j s_j z_j and Q = sum_j s_j z_j^2 by the reduction tree of ses_update_openai (rows sharded over the
+ *                 attached peers likewise); then p_sigma, h_sigma = (|p_sigma| < threshold), m (old sigma, old c), p_c, c and sigma
+ *                 as section 4.11 writes them; parent_dev [D] f32 := (float)m.  1 <= mu <= population. */
+typedef struct ses_cma_params {
+    double one_m_cs;   /* 1 - c_sigma                          */
+    double k_sigma;    /* sqrt(c_sigma (2 - c_sigma) mu_eff)   */
+    double one_m_cc;   /* 1 - c_c                              */
+    double k_c;        /* sqrt(c_c (2 - c_c) mu_eff)           */
+    double cc2;        /* c_c (2 - c_c)                        */
+    double c_keep;     /* 1 - c_1 - c_mu                       */
+    double c1;         /* c_1 (separable rescaling applied)    */
+    double cmu;        /* c_mu (separable rescaling applied)   */
+    double damp;       /* c_sigma / d_sigma                    */
+    double chi;        /* E|N(0, I_D)|: chi_D                  */
+} ses_cma_params;
+int ses_cma_sample(ses_handle *h, uint32_t generation, const double *mean_dev, const double *c_dev, const double *sigma_dev,
+                   float *out_dev, void *stream);
+int ses_cma_update(ses_handle *h, uint32_t generation, const int32_t *order_dev, const double *weights_dev, int32_t mu,
+                   const ses_cma_params *params, double threshold, double *s_dev, double *mean_dev, double *c_dev,
+                   double *p_sigma_dev, double *p_c_dev, double *sigma_dev, float *parent_dev, void *stream);
 
 /* Number of kernels this library has launched on behalf of the handle (bench.py "gpu_launches"). */
 int64_t ses_launch_count(ses_handle *h);

@@ -13,7 +13,7 @@ TEST_LIB_PATH = os.path.join(_PKG, "libses_b200_tests.so")
 SOURCES = [os.path.join(_PKG, "csrc", f) for f in (
     "ses_abi.cu", "ses_common.cuh", "rollout_slots.cuh", "rollout_cartpole_mlp.cuh", "rollout_cartpole_gru.cuh", "rollout_mpe.cuh",
     "rollout_classic.cuh", "rollout_gru_generic.cuh",
-    "rank.cuh", "update.cuh", "novelty.cuh")]
+    "rank.cuh", "update.cuh", "novelty.cuh", "cma.cuh")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-fmad=false",           # numerical contract: FMAs only where written (DESIGN.md section 4)
               "-Xcompiler", "-fPIC", "-shared"]
@@ -24,6 +24,10 @@ class ses_config(C.Structure):
         "env", "obs_dim", "act_dim", "gru", "pomdp", "n_agents", "max_step", "eval_ep_num", "population", "group",
         "n_head", "n_parents")] + [("seed", C.c_uint32)] + [(n, C.c_int32) for n in (
             "init_mode", "id_begin", "id_end", "device", "antithetic", "shard_block", "shard_rank", "shard_world", "continuous_action")] + [("reserved", C.c_int32 * 2)]
+
+
+class ses_cma_params(C.Structure):
+    _fields_ = [(n, C.c_double) for n in ("one_m_cs", "k_sigma", "one_m_cc", "k_c", "cc2", "c_keep", "c1", "cmu", "damp", "chi")]
 
 
 # every symbol include/ses_b200.h declares: name -> (restype, argtypes)
@@ -58,6 +62,8 @@ SYMBOLS = {
     "ses_behavior": (C.c_int, [_vp, _vp, _i32, _vp, _vp]),
     "ses_novelty": (C.c_int, [_vp, _vp, _i32, _vp, _i32, _i32, _vp, _vp]),
     "ses_blend_shaped": (C.c_int, [_vp, _vp, _vp, _i32, _f64, _vp, _vp]),
+    "ses_cma_sample": (C.c_int, [_vp, _u32, _vp, _vp, _vp, _vp, _vp]),
+    "ses_cma_update": (C.c_int, [_vp, _u32, _vp, _vp, _i32, C.POINTER(ses_cma_params), _f64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
 }
 # include/ses_b200_test.h: only in the test build
 TEST_SYMBOLS = {

@@ -14,6 +14,7 @@
 #include <cstdlib>
 #include <cstring>
 
+#include "cma.cuh"
 #include "novelty.cuh"
 #include "rank.cuh"
 #include "rollout_cartpole_mlp.cuh"
@@ -222,7 +223,7 @@ extern "C" int ses_create(const ses_config *cfg, ses_handle **out)
     CU(cudaMalloc(&h->hist, sizeof(int) * h->n_tiles * 256));
     CU(cudaMalloc(&h->tot, sizeof(int) * 8 * 256));
     CU(cudaMalloc(&h->hist_fused, sizeof(int) * (8 * (size_t)h->n_tiles * 256 + 1)));   // + the persistent kernel's grid-barrier counter
-    CU(cudaMalloc(&h->part1, sizeof(double) * (size_t)h->nb1 * h->DP));
+    CU(cudaMalloc(&h->part1, sizeof(double) * 2 * (size_t)h->nb1 * h->DP));     // two tables: k_grad_partial<true> (sep_cma_es)
     *out = h;
     return 0;
 }
@@ -649,7 +650,8 @@ extern "C" int ses_blend_shaped(ses_handle *h, const double *shaped_f_dev, const
 // ------------------------------------------------------------------------------------------------
 // peer fitness exchange (multi-GPU): IPC-mapped exchange buffers + a flag barrier over NVLink
 // ------------------------------------------------------------------------------------------------
-static size_t xbuf_doubles(const ses_handle *h) { return 2 * (size_t)h->cfg.population + 2 * MAX_PEERS + (size_t)h->nb1 * h->DP; }
+// [2][P] fitness, flags, then the gradient rows: two [nb1][DP] tables (the second one only for sep_cma_es's k_grad_partial<true>)
+static size_t xbuf_doubles(const ses_handle *h) { return 2 * (size_t)h->cfg.population + 2 * MAX_PEERS + 2 * (size_t)h->nb1 * h->DP; }
 static double *xbuf_part1(double *base, const ses_handle *h) { return base + 2 * (size_t)h->cfg.population + 2 * MAX_PEERS; }
 static unsigned long long *xbuf_flags(double *base, const ses_handle *h) { return reinterpret_cast<unsigned long long *>(base + 2 * (size_t)h->cfg.population); }
 
@@ -865,9 +867,10 @@ extern "C" int ses_rank_desc(ses_handle *h, const double *fitness_dev, int32_t n
 // K3
 // ------------------------------------------------------------------------------------------------
 // levels 0 + 1 of the gradient (k_grad_partial, and the peer barrier when the rows are sharded over ranks);
-// *part1_out is the [nb1][DP] table the level-2 kernels read
+// *part1_out is the [nb1][DP] table the level-2 kernels read.  sq: k_grad_partial<true>, whose second table (the squared
+// noise) follows at *part1_out + nb1 * DP
 static int grad_levels01(ses_handle *h, uint32_t generation, const double *shaped_dev, const float *eps_override_dev,
-                         void *stream, double **part1_out)
+                         void *stream, double **part1_out, bool sq = false)
 {
     cudaStream_t st = S(stream);
     const int P = h->cfg.population;
@@ -896,8 +899,9 @@ static int grad_levels01(ses_handle *h, uint32_t generation, const double *shape
         sync.expected = (g1 - g0) * n_chunks;
     }
     if (g1 > g0) {
-        k_grad_partial<<<(g1 - g0) * n_chunks, GB1 * GQC, 0, st>>>(shaped_dev, P, h->D, h->NQ, h->cfg.seed, generation, lay, eps_override_dev,
-                                                                  part1, h->nb0, g0, n_chunks, n_peers, peers, sync);
+        auto kernel = sq ? k_grad_partial<true> : k_grad_partial<false>;
+        kernel<<<(g1 - g0) * n_chunks, GB1 * GQC, 0, st>>>(shaped_dev, P, h->D, h->NQ, h->cfg.seed, generation, lay, eps_override_dev,
+                                                          part1, h->nb0, g0, n_chunks, n_peers, peers, sync);
         h->launches += 1;
     }
     if (shard && !fold && peer_barrier_launch(h, stream, nullptr)) return -1;
@@ -937,6 +941,58 @@ extern "C" int ses_update_openai_sgd(ses_handle *h, uint32_t generation, const d
     if (grad_levels01(h, generation, shaped_dev, eps_override_dev, stream, &part1)) return -1;
     k_grad_final_sgd<<<(h->D + 255) / 256, 256, 0, st>>>(part1, h->nb1, h->DP, h->D, (float)update_factor, (float)(-stepsize),
                                                         (float)momentum, (float)(1.0 - momentum), mu_dev, v_dev, grad_out_dev);
+    h->launches += 1;
+    CU(cudaGetLastError());
+    return 0;
+}
+
+// ------------------------------------------------------------------------------------------------
+// sep_cma_es (DESIGN.md section 4.11)
+// ------------------------------------------------------------------------------------------------
+static int cma_layout_ok(const ses_handle *h, const char *fn)
+{
+    if (h->cfg.group != h->cfg.population || h->cfg.n_head != 0 || h->cfg.antithetic)
+        return fail("%s: needs the sep_cma_es layout (group = population, n_head = 0, no antithetic pairs); this handle has group %d, "
+                    "n_head %d, antithetic %d", fn, h->cfg.group, h->cfg.n_head, h->cfg.antithetic);
+    return 0;
+}
+
+extern "C" int ses_cma_sample(ses_handle *h, uint32_t generation, const double *mean_dev, const double *c_dev, const double *sigma_dev,
+                              float *out_dev, void *stream)
+{
+    if (!h) return fail("ses_cma_sample: null handle");
+    if (!mean_dev || !c_dev || !sigma_dev || !out_dev) return fail("ses_cma_sample: mean_dev, c_dev, sigma_dev and out_dev are required");
+    if (cma_layout_ok(h, "ses_cma_sample")) return -1;
+    if (h->shard.n_local == 0) return 0;
+    CU(cudaSetDevice(h->cfg.device));
+    const long long total = (long long)h->shard.n_local * h->NQ;
+    k_cma_sample<<<(unsigned)((total + 255) / 256), 256, 0, S(stream)>>>(mean_dev, c_dev, sigma_dev, h->shard, h->D, h->NQ, h->cfg.seed,
+                                                                          generation, out_dev);
+    CU(cudaGetLastError());
+    h->launches += 1;
+    return 0;
+}
+
+extern "C" int ses_cma_update(ses_handle *h, uint32_t generation, const int32_t *order_dev, const double *weights_dev, int32_t mu,
+                              const ses_cma_params *params, double threshold, double *s_dev, double *mean_dev, double *c_dev,
+                              double *p_sigma_dev, double *p_c_dev, double *sigma_dev, float *parent_dev, void *stream)
+{
+    if (!h) return fail("ses_cma_update: null handle");
+    if (!order_dev || !weights_dev || !params || !s_dev || !mean_dev || !c_dev || !p_sigma_dev || !p_c_dev || !sigma_dev || !parent_dev)
+        return fail("ses_cma_update: null argument");
+    if (cma_layout_ok(h, "ses_cma_update")) return -1;
+    const int P = h->cfg.population;
+    if (mu < 1 || mu > P) return fail("ses_cma_update: mu=%d outside [1, population=%d]", mu, P);
+    CU(cudaSetDevice(h->cfg.device));
+    cudaStream_t st = S(stream);
+    k_cma_weights<<<(P + 255) / 256, 256, 0, st>>>(order_dev, weights_dev, mu, P, s_dev);
+    h->launches += 1;
+    double *part1 = nullptr;
+    if (grad_levels01(h, generation, s_dev, nullptr, stream, &part1, true)) return -1;
+    const CmaParams pr{params->one_m_cs, params->k_sigma, params->one_m_cc, params->k_c, params->cc2, params->c_keep, params->c1,
+                       params->cmu, params->damp, params->chi};
+    k_cma_final<<<1, CMA_THREADS, 0, st>>>(part1, h->nb1, h->DP, h->D, pr, threshold, mean_dev, c_dev, p_sigma_dev, p_c_dev, sigma_dev,
+                                           parent_dev);
     h->launches += 1;
     CU(cudaGetLastError());
     return 0;

@@ -28,20 +28,28 @@ constexpr int GQC = 2;
 // shared memory and are added sequentially in block order (level 1).  part1[g][DP] float64.
 // Groups [g_begin, g_end) only: with several ranks each computes its share of the groups and stores the rows
 // into every peer's part1 buffer over NVLink (peer_part1), so that all ranks finish with the same table.
+// SQ (sep_cma_es, DESIGN.md section 4.11): a second table of sum_j shaped_j eps_jd^2 (eps^2 formed exactly in float64) in the
+// same pass, at part1 + nb1 * DP, mirrored to the peers likewise.  Rows with shaped_j == 0 are skipped: their fma would add
+// an exact zero to a sum that is never -0.0, so both tables keep their bits.
+template <bool SQ = false>
 __global__ void __launch_bounds__(GB1 * GQC) k_grad_partial(const double *__restrict__ shaped, int P, int D, int NQ, uint32_t seed,
                                                             uint32_t gen, Layout layout, const float *__restrict__ eps_override,
                                                             double *__restrict__ part1, int nb0, int g_begin, int n_chunks,
                                                             int n_peers, PeerRows peers, const PeerSync sync)
 {
-    __shared__ double sp[GB1][GQC * 4];
+    __shared__ double sp[SQ ? 2 : 1][GB1][GQC * 4];
     const int g = g_begin + blockIdx.x / n_chunks;
     const int qc = blockIdx.x % n_chunks;
     const int bb = threadIdx.x / GQC, qq = threadIdx.x % GQC;
     const int b = g * GB1 + bb, q = qc * GQC + qq;
     double a0 = 0.0, a1 = 0.0, a2 = 0.0, a3 = 0.0;
+    [[maybe_unused]] double s0 = 0.0, s1 = 0.0, s2 = 0.0, s3 = 0.0;
     if (b < nb0 && q < NQ) {
         const int j1 = min(P, (b + 1) * GB0);
         for (int j = b * GB0; j < j1; ++j) {
+            if constexpr (SQ) {
+                if (shaped[j] == 0.0) continue;
+            }
             float4 e;
             if (eps_override) {
                 const float *row = eps_override + (size_t)j * D;
@@ -62,19 +70,35 @@ __global__ void __launch_bounds__(GB1 * GQC) k_grad_partial(const double *__rest
             a1 = fma((double)e.y, f, a1);
             a2 = fma((double)e.z, f, a2);
             a3 = fma((double)e.w, f, a3);
+            if constexpr (SQ) {
+                s0 = fma(__dmul_rn((double)e.x, (double)e.x), f, s0);
+                s1 = fma(__dmul_rn((double)e.y, (double)e.y), f, s1);
+                s2 = fma(__dmul_rn((double)e.z, (double)e.z), f, s2);
+                s3 = fma(__dmul_rn((double)e.w, (double)e.w), f, s3);
+            }
         }
     }
-    sp[bb][qq * 4 + 0] = a0; sp[bb][qq * 4 + 1] = a1; sp[bb][qq * 4 + 2] = a2; sp[bb][qq * 4 + 3] = a3;
+    sp[0][bb][qq * 4 + 0] = a0; sp[0][bb][qq * 4 + 1] = a1; sp[0][bb][qq * 4 + 2] = a2; sp[0][bb][qq * 4 + 3] = a3;
+    if constexpr (SQ) {
+        sp[1][bb][qq * 4 + 0] = s0; sp[1][bb][qq * 4 + 1] = s1; sp[1][bb][qq * 4 + 2] = s2; sp[1][bb][qq * 4 + 3] = s3;
+    }
     __syncthreads();
     if (threadIdx.x < GQC * 4) {
         const int d = qc * GQC * 4 + threadIdx.x;
         if (d < NQ * 4) {
             const int nb = min(GB1, nb0 - g * GB1);
             double t = 0.0;
-            for (int k = 0; k < nb; ++k) t = __dadd_rn(t, sp[k][threadIdx.x]);
+            for (int k = 0; k < nb; ++k) t = __dadd_rn(t, sp[0][k][threadIdx.x]);
             const size_t o = (size_t)g * (NQ * 4) + d;
             part1[o] = t;
             for (int r = 0; r < n_peers; ++r) peers.p[r][o] = t;
+            if constexpr (SQ) {
+                double t2 = 0.0;
+                for (int k = 0; k < nb; ++k) t2 = __dadd_rn(t2, sp[1][k][threadIdx.x]);
+                const size_t o2 = o + (size_t)((nb0 + GB1 - 1) / GB1) * (NQ * 4);      // + nb1 * DP: the second table
+                part1[o2] = t2;
+                for (int r = 0; r < n_peers; ++r) peers.p[r][o2] = t2;
+            }
         }
         if (n_peers > 0) __threadfence_system();                   // the rows before this CTA's arrival below
     }

@@ -38,6 +38,8 @@ def population_layout(strategy, offspring_num, elite_num=None):
         return n + 1, n + 1, 2, 1            # [mu, elite0 (== mu), n-1 perturbed]
     if strategy in ("openai_es", "nsr_es"):
         return n, n, 1, 1                    # [mu, n-1 perturbed]
+    if strategy == "sep_cma_es":
+        return n, n, 0, 1                    # every offspring sampled (DESIGN.md section 4.11)
     if strategy == "simple_genetic":
         k = int(elite_num)
         g = n // k
@@ -45,6 +47,36 @@ def population_layout(strategy, offspring_num, elite_num=None):
             raise ValueError("simple_genetic needs offspring_num >= elite_num")
         return k * g, g, 1, k                # per elite: [elite, g-1 perturbed]
     raise ValueError("unknown strategy %r" % (strategy,))
+
+
+def sep_cma_constants(D, lam, mu):
+    """Host constants of sep_cma_es (DESIGN.md section 4.11; Hansen's defaults with the separable rescaling of Ros & Hansen
+    2008), float64: the recombination weights [mu], the learning rates, and the fields of ses_cma_params."""
+    D, lam, mu = int(D), int(lam), int(mu)
+    if not 1 <= mu <= lam:
+        raise ValueError("sep_cma_es needs 1 <= elite_num <= offspring_num (got %d, %d)" % (mu, lam))
+    w = np.log(mu + 0.5) - np.log(np.arange(1, mu + 1, dtype=np.float64))
+    w = w / w.sum()
+    mu_eff = 1.0 / float(np.sum(w * w))
+    c_sigma = (mu_eff + 2.0) / (D + mu_eff + 5.0)
+    d_sigma = 1.0 + 2.0 * max(0.0, math.sqrt((mu_eff - 1.0) / (D + 1.0)) - 1.0) + c_sigma
+    c_c = (4.0 + mu_eff / D) / (D + 4.0 + 2.0 * mu_eff / D)
+    c1 = 2.0 / ((D + 1.3) ** 2 + mu_eff)
+    cmu = min(1.0 - c1, 2.0 * (mu_eff - 2.0 + 1.0 / mu_eff) / ((D + 2.0) ** 2 + mu_eff))
+    c1 = c1 * (D + 2.0) / 3.0
+    cmu = min(1.0 - c1, cmu * (D + 2.0) / 3.0)
+    chi = math.sqrt(D) * (1.0 - 1.0 / (4.0 * D) + 1.0 / (21.0 * D * D))
+    return {"weights": w, "mu": mu, "mu_eff": mu_eff, "c_sigma": c_sigma, "d_sigma": d_sigma, "c_c": c_c, "c1": c1, "cmu": cmu,
+            "chi": chi, "D": D,
+            "one_m_cs": 1.0 - c_sigma, "k_sigma": math.sqrt(c_sigma * (2.0 - c_sigma) * mu_eff), "one_m_cc": 1.0 - c_c,
+            "k_c": math.sqrt(c_c * (2.0 - c_c) * mu_eff), "cc2": c_c * (2.0 - c_c), "c_keep": 1.0 - c1 - cmu,
+            "damp": c_sigma / d_sigma}
+
+
+def sep_cma_threshold(k, generation):
+    """h_sigma's threshold T_g of generation g (0-based) for the constants k of sep_cma_constants."""
+    D = k["D"]
+    return (1.4 + 2.0 / (D + 1.0)) * k["chi"] * math.sqrt(1.0 - (1.0 - k["c_sigma"]) ** (2 * (int(generation) + 1)))
 
 
 def shard_bounds(P, rank, world):
@@ -65,6 +97,11 @@ def owned_ids(P, rank, world, block):
     blocks = np.arange(rank, (P + block - 1) // block, world, dtype=np.int64)
     ids = (blocks[:, None] * block + np.arange(block, dtype=np.int64)[None, :]).reshape(-1)
     return ids[ids < P]
+
+
+def cma_params(k):
+    """The ses_cma_params struct of sep_cma_constants(...) k."""
+    return C.byref(_lib.ses_cma_params(**{f: float(k[f]) for f, _ in _lib.ses_cma_params._fields_}))
 
 
 def _ptr(t):
@@ -233,6 +270,33 @@ class RolloutEngine:
         self._chk(out, torch.float64, n, "out")
         self._check(self.lib.ses_blend_shaped(self._h, _ptr(shaped_f), _ptr(shaped_n), n, float(w), _ptr(out), self._stream()))
         return out
+
+    # ------------------------------------------------------------------------------ sep_cma_es
+    def cma_sample(self, generation, mean, c, sigma, out=None):
+        """Step 1 of sep_cma_es (DESIGN.md section 4.11): [n_local, D] f32, row l = (float)(mean + sigma (sqrt(c) z)) for the
+        l-th id this engine owns, in rollout()'s w_override order.  mean, c: [D] f64; sigma: [1] f64 (all CUDA tensors)."""
+        self._chk(mean, torch.float64, self.D, "mean")
+        self._chk(c, torch.float64, self.D, "c")
+        self._chk(sigma, torch.float64, 1, "sigma")
+        if out is None:
+            out = torch.empty((self.n_local, self.D), dtype=torch.float32, device=self.device)
+        self._chk(out, torch.float32, self.n_local * self.D, "out")
+        self._check(self.lib.ses_cma_sample(self._h, int(generation), _ptr(mean), _ptr(c), _ptr(sigma), _ptr(out), self._stream()))
+        return out
+
+    def cma_update(self, generation, order, consts, weights, s, mean, c, p_sigma, p_c, sigma, parent):
+        """Steps 3-5 of sep_cma_es in place: s [P] f64 := the recombination weight of every id (weights [mu] f64 at order[:mu]),
+        then mean, c, p_sigma, p_c ([D] f64), sigma ([1] f64) and parent ([D] f32 := mean).  `consts`: sep_cma_constants."""
+        self._chk(order, torch.int32, self.P, "order")
+        self._chk(weights, torch.float64, int(consts["mu"]), "weights")
+        self._chk(s, torch.float64, self.P, "s")
+        for name, x in (("mean", mean), ("c", c), ("p_sigma", p_sigma), ("p_c", p_c)):
+            self._chk(x, torch.float64, self.D, name)
+        self._chk(sigma, torch.float64, 1, "sigma")
+        self._chk(parent, torch.float32, self.D, "parent")
+        self._check(self.lib.ses_cma_update(self._h, int(generation), _ptr(order), _ptr(weights), int(consts["mu"]), cma_params(consts),
+                                            sep_cma_threshold(consts, generation), _ptr(s), _ptr(mean), _ptr(c), _ptr(p_sigma),
+                                            _ptr(p_c), _ptr(sigma), _ptr(parent), self._stream()))
 
     # ------------------------------------------------------------------------------ K1
     def rollout(self, generation, sigma, parents, fitness=None, steps=None, w_override=None, init_states=None,

@@ -1,5 +1,5 @@
-"""Device-resident strategy state for the offspring strategies: the reference's three, and nsr_es (novelty search with
-reward), an opt-in addition.
+"""Device-resident strategy state for the offspring strategies: the reference's three, and two opt-in additions: nsr_es
+(novelty search with reward) and sep_cma_es (separable CMA-ES).
 
 Each class keeps what the reference strategy keeps (learning_strategies/evolution/offspring_strategies.py)
 -- mu / elite table, sigma, Adam moments -- as a few small CUDA tensors, and never materialises the
@@ -10,7 +10,7 @@ generation: K1 rollout of this rank's slice, fitness exchange, K2 rank, K3 updat
 import torch
 
 from . import dist as sdist
-from .engine import RolloutEngine, cyclic_block, owned_ids, population_layout, shard_bounds
+from .engine import RolloutEngine, cyclic_block, owned_ids, population_layout, sep_cma_constants, shard_bounds
 
 
 class _Base:
@@ -335,4 +335,95 @@ class NoveltyES(OpenAIES):
         self.n_archive = int(a.shape[0])
 
 
-STRATEGIES = {c.name: c for c in (OpenAIES, SimpleEvolution, SimpleGenetic, NoveltyES)}
+def _cma_params(cfg):
+    """(offspring_num, elite_num, init_sigma) of a sep_cma_es strategy section, validated."""
+    allowed = {"name", "init_sigma", "offspring_num", "elite_num"}
+    unknown = sorted(set(cfg) - allowed)
+    if unknown:
+        raise ValueError("strategy sep_cma_es: unknown key(s) %s (allowed: %s)" % (", ".join(unknown), ", ".join(sorted(allowed))))
+    sigma, lam = cfg.get("init_sigma"), cfg.get("offspring_num")
+    if isinstance(sigma, bool) or not isinstance(sigma, (int, float)) or not float(sigma) > 0.0 or sigma == float("inf"):
+        raise ValueError("strategy sep_cma_es: init_sigma must be a finite number > 0 (got %r)" % (sigma,))
+    if isinstance(lam, bool) or not isinstance(lam, int) or lam < 2:
+        raise ValueError("strategy sep_cma_es: offspring_num must be an integer >= 2 (got %r)" % (lam,))
+    mu = cfg.get("elite_num", lam // 2)
+    if isinstance(mu, bool) or not isinstance(mu, int) or not 1 <= mu <= lam:
+        raise ValueError("strategy sep_cma_es: elite_num must be an integer in [1, offspring_num = %d] (got %r)" % (lam, mu))
+    return lam, mu, float(sigma)
+
+
+class SepCMAES(_Base):
+    """Separable CMA-ES (Ros & Hansen 2008; opt-in, the reference has no such strategy): every offspring is drawn from
+    N(m, sigma^2 diag(c)), and the mu best recombine into the new mean, the evolution paths, the diagonal c and sigma.  The
+    state (m, c, p_sigma, p_c, sigma) is float64 and lives on the device; the samples are the w_override table K1 rolls out
+    (DESIGN.md section 4.11)."""
+    name = "sep_cma_es"
+
+    def __init__(self, strategy_cfg, env_cfg, network_cfg, eval_ep_num, seed, device, engine_cfg):
+        lam, mu, sigma = _cma_params(strategy_cfg)
+        if engine_cfg.get("antithetic", False):
+            raise ValueError("sep_cma_es does not support engine.antithetic: mirrored samples bias its step-size adaptation")
+        super().__init__(dict(strategy_cfg, sigma_decay=1.0, elite_num=mu), env_cfg, network_cfg, eval_ep_num, seed, device, engine_cfg)
+        dev = self.engine.device
+        self.mu = mu
+        self.consts = sep_cma_constants(self.D, self.P, mu)
+        self._run_key.update(elite_num=mu)
+        self.weights = torch.from_numpy(self.consts["weights"]).to(dev)
+        self.mean = torch.zeros(self.D, dtype=torch.float64, device=dev)
+        self.c = torch.ones(self.D, dtype=torch.float64, device=dev)
+        self.p_sigma = torch.zeros(self.D, dtype=torch.float64, device=dev)
+        self.p_c = torch.zeros(self.D, dtype=torch.float64, device=dev)
+        self.sigma_dev = torch.full((1,), sigma, dtype=torch.float64, device=dev)
+        self.s = torch.empty(self.P, dtype=torch.float64, device=dev)
+        self.samples = torch.empty((self.engine.n_local, self.D), dtype=torch.float32, device=dev)
+
+    @property
+    def curr_sigma(self):
+        """sigma of the next generation: the device value (B200Loop reads it after its one sync per generation)."""
+        return float(self.sigma_dev.item()) if hasattr(self, "sigma_dev") else self.sigma
+
+    @curr_sigma.setter
+    def curr_sigma(self, value):
+        if hasattr(self, "sigma_dev"):
+            self.sigma_dev.fill_(float(value))
+
+    def step(self):
+        e = self.engine
+        self._mark(0)
+        e.cma_sample(self.generation, self.mean, self.c, self.sigma_dev, out=self.samples)
+        self.fitness = self._fit[self.generation & 1]
+        e.rollout(self.generation, 0.0, self.parents, fitness=self.fitness, steps=self.steps, w_override=self.samples)
+        self.exchange_fitness()
+        self._mark(1)
+        e.rank_desc(self.fitness, order=self.order)
+        e.cma_update(self.generation, self.order, self.consts, self.weights, self.s, self.mean, self.c, self.p_sigma, self.p_c,
+                     self.sigma_dev, self.parents[0])
+        self.generation += 1
+        self._mark(2)
+
+    def elite_flat(self):
+        return self.parents[0]                                    # (float)m, written by every update
+
+    def load_elite(self, flat):
+        """Start from a saved policy: m := flat, c := 1, both paths := 0 (sigma stays init_sigma)."""
+        super().load_elite(flat)
+        self.mean.copy_(self.parents[0].double())
+        self.c.fill_(1.0)
+        self.p_sigma.zero_()
+        self.p_c.zero_()
+
+    def state(self):
+        st = super().state()
+        for k in ("mean", "c", "p_sigma", "p_c", "sigma_dev"):
+            st[k] = getattr(self, k).detach().cpu().clone()
+        return st
+
+    def load_state(self, st):
+        super().load_state(st)
+        for k in ("mean", "c", "p_sigma", "p_c", "sigma_dev"):
+            if tuple(st[k].shape) != tuple(getattr(self, k).shape):
+                raise ValueError("resume state has %s of shape %s, this run needs %s" % (k, tuple(st[k].shape), tuple(getattr(self, k).shape)))
+            getattr(self, k).copy_(st[k])
+
+
+STRATEGIES = {c.name: c for c in (OpenAIES, SimpleEvolution, SimpleGenetic, NoveltyES, SepCMAES)}
