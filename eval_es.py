@@ -10,6 +10,10 @@ one call on the same episodes: episode m starts from the env's reset distributio
 compared on identical initial states.  One line per checkpoint; --out writes returns [n_ckpt, episodes] (float64), lengths
 [n_ckpt, episodes] (int32) and the checkpoint paths to an .npz file.
 
+--archive PATH evaluates every elite of a map_elites archive file (archive_ep_<n>.pt, as B200Loop saves it) in one call
+instead of checkpoints: one summary line, and --out writes returns / lengths [n_elites, episodes] with the archive's cells.
+An elite's fitness in the archive comes from the eval_ep_num training episodes of its generation; this re-scores it.
+
 --record K also records the first K of those episodes step by step and adds them to --out: initial [K, state_dim] (the
 initial states), states [n_ckpt, K, T, state_dim] (the state after each step; for the gym envs their env.unwrapped.state, so
 a gym install can replay them into its renderer), actions [n_ckpt, K, T, n_agents], step_returns [n_ckpt, K, T] (the return
@@ -25,7 +29,9 @@ import yaml
 def parse_args(argv=None):
     ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
     ap.add_argument("--cfg-path", required=True, help="training config (its env and network sections are used).")
-    ap.add_argument("--ckpt-path", required=True, nargs="+", help="GymEnvModel state_dict(s) to evaluate.")
+    src = ap.add_mutually_exclusive_group(required=True)
+    src.add_argument("--ckpt-path", nargs="+", help="GymEnvModel state_dict(s) to evaluate.")
+    src.add_argument("--archive", default=None, help="a map_elites archive file (archive_ep_<n>.pt): evaluate every elite.")
     ap.add_argument("--episodes", type=int, default=100, help="episodes per checkpoint (test.py runs 100).")
     ap.add_argument("--seed", type=int, default=0, help="seed of the initial states.")
     ap.add_argument("--round", type=int, default=0, help="another set of initial states under the same seed.")
@@ -37,6 +43,8 @@ def parse_args(argv=None):
     if args.episodes < 1:
         ap.error("--episodes must be >= 1")
     if args.record is not None:
+        if args.archive:
+            ap.error("--record takes checkpoints (--ckpt-path), not --archive")
         if not args.out:
             ap.error("--record needs --out")
         if not 1 <= args.record <= args.episodes:
@@ -71,17 +79,46 @@ def load_policies(paths, obs_dim, act_dim, gru):
     return torch.stack(flats)
 
 
+def load_archive(path, obs_dim, act_dim, gru):
+    """(weights [n_elites, D] float32 CPU, cells [n_elites] int64) of a map_elites archive file."""
+    import torch
+
+    from simple_es_b200 import checkpoint
+    a = torch.load(path, map_location="cpu")
+    if not isinstance(a, dict) or "weights" not in a or "cells" not in a:
+        raise ValueError("%s is not a map_elites archive file (archive_ep_<n>.pt)" % path)
+    D = sum(int(np.prod(shape)) for _, shape in checkpoint.param_shapes(obs_dim, act_dim, gru))
+    W = torch.as_tensor(a["weights"], dtype=torch.float32)
+    if W.dim() != 2 or W.shape[1] != D:
+        raise ValueError("%s holds weights of shape %s; the config's network has %d parameters" % (path, tuple(W.shape), D))
+    if W.shape[0] == 0:
+        raise ValueError("%s holds an empty archive" % path)
+    return W, torch.as_tensor(a["cells"], dtype=torch.int64)
+
+
 def main(argv=None):
     args = parse_args(argv)
     with open(args.cfg_path) as fh:
         config = yaml.load(fh, Loader=yaml.FullLoader)
     kw = engine_config(config)
-    W = load_policies(args.ckpt_path, kw["obs_dim"], kw["act_dim"], kw["gru"])
+    if args.archive:
+        W, cells = load_archive(args.archive, kw["obs_dim"], kw["act_dim"], kw["gru"])
+    else:
+        W = load_policies(args.ckpt_path, kw["obs_dim"], kw["act_dim"], kw["gru"])
     from simple_es_b200.engine import RolloutEngine
     # the population layout of the handle plays no part in an evaluation: the smallest valid one
     eng = RolloutEngine(eval_ep_num=1, population=2, group=2, n_head=1, n_parents=1, seed=args.seed, device=args.device, **kw)
     ret, lng = eng.evaluate(W.to(eng.device), args.episodes, round=args.round)
     ret, lng = ret.cpu().numpy(), lng.cpu().numpy()
+    if args.archive:
+        means = ret.mean(axis=1)
+        b = int(np.argmax(means))
+        print(f"{args.archive}: {ret.shape[0]} elites x {ret.shape[1]} episodes, mean of elite means {means.mean():.2f}, "
+              f"best elite cell {int(cells[b])} mean {means[b]:.2f}, worst elite mean {means.min():.2f}")
+        if args.out:
+            np.savez(args.out, returns=ret, lengths=lng, cells=cells.numpy(), archive=np.array(args.archive))
+        eng.close()
+        return ret, lng
     for path, r, n in zip(args.ckpt_path, ret, lng):
         print(f"{path}: {r.size} episodes, mean {r.mean():.2f}, std {r.std():.2f}, min {r.min():.2f}, max {r.max():.2f}, "
               f"mean length {n.mean():.1f}")

@@ -256,6 +256,40 @@ int ses_cma_update(ses_handle *h, uint32_t generation, const int32_t *order_dev,
                    const ses_cma_params *params, double threshold, double *s_dev, double *mean_dev, double *c_dev,
                    double *p_sigma_dev, double *p_c_dev, double *sigma_dev, float *parent_dev, void *stream);
 
+/* MAP-Elites (the map_elites strategy, DESIGN.md section 4.12; Mouret & Clune 2015).  Needs the layout group = 1, n_head = 0,
+ * antithetic = 0 (n_parents = population): offspring i is parent row i + sigma * its Philox noise.  The archive has
+ * n_cells = prod cells[j] cells, every buffer a caller-owned device array indexed by cell c:
+ *   F_dev [n_cells] f64 the elite's fitness; NaN marks an empty cell (fill with NaN before the first call)
+ *   B_dev [n_cells][state_dim] f64 its behaviour;  born_dev [n_cells][2] i32 its (generation, offspring id);  W_dev [n_cells][D] f32
+ *   its weights.
+ * The spec picks n_dims in [1, 4] distinct final-state coordinates dims[j] in [0, state_dim) with finite low[j], finite
+ * width[j] = high - low > 0 (computed by the caller in float64) and cells[j] >= 1; n_cells <= 2^20 and n_cells * D * 4 bytes
+ * <= 4 GiB.  Cell of a behaviour row b: per dimension s = ((b[dims[j]] - low) / width) * cells (float64, each operation
+ * rounded), k = 0 if s < 1, cells - 1 if s >= cells - 1, floor(s) otherwise; c is row-major over the dimensions.
+ * ses_map_insert: reads parents_dev [population][D] f32 (the table the generation was rolled out with), order_dev [population]
+ *                 (ses_rank_desc of the full fitness vector), fitness_dev [population] f64 and bc_dev [population][state_dim]
+ *                 f64 (ses_behavior).  An offspring whose fitness or a descriptor coordinate is NaN is unplaced; each cell's
+ *                 placed offspring of smallest rank enters iff the cell is empty or its fitness > F (a tie keeps the incumbent),
+ *                 writing F, B, born = (generation, id) and W = its weights (those of ses_materialize(generation, sigma)).
+ * ses_map_select: from F_dev and W_dev: stats_dev [4] f64 := (n_occ, best cell c* (largest F, ties to the lowest index; -1
+ *                 when empty), F[c*] (NaN when empty), the QD score sum of F over occupied cells in section 4.12's order); then
+ *                 parent row i of parents_dev [population][D] := W[L[(r_i * n_occ) >> 32]], L the occupied cells ascending and
+ *                 r_i word 0 of Philox(i, generation, 0, 0; seed, 3), or seed_row_dev [D] f32 when the archive is empty.
+ * Both refuse null buffers, a bad spec and another layout.  Only the first call, and one with more cells than any before,
+ * waits for the stream: it allocates the handle's scratch (per-cell claims, zero between calls, and the occupied-cell list). */
+typedef struct ses_map_spec {
+    int32_t n_dims;
+    int32_t dims[4];
+    double low[4];
+    double width[4];
+    int32_t cells[4];
+} ses_map_spec;
+int ses_map_insert(ses_handle *h, uint32_t generation, float sigma, const float *parents_dev, const int32_t *order_dev,
+                   const double *fitness_dev, const double *bc_dev, const ses_map_spec *spec, double *F_dev, double *B_dev,
+                   int32_t *born_dev, float *W_dev, void *stream);
+int ses_map_select(ses_handle *h, uint32_t generation, const ses_map_spec *spec, const double *F_dev, const float *W_dev,
+                   const float *seed_row_dev, double *stats_dev, float *parents_dev, void *stream);
+
 /* Number of kernels this library has launched on behalf of the handle (bench.py "gpu_launches"). */
 int64_t ses_launch_count(ses_handle *h);
 

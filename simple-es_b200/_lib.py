@@ -13,7 +13,7 @@ TEST_LIB_PATH = os.path.join(_PKG, "libses_b200_tests.so")
 SOURCES = [os.path.join(_PKG, "csrc", f) for f in (
     "ses_abi.cu", "ses_common.cuh", "rollout_slots.cuh", "rollout_cartpole_mlp.cuh", "rollout_cartpole_gru.cuh", "rollout_mpe.cuh",
     "rollout_classic.cuh", "rollout_gru_generic.cuh",
-    "rank.cuh", "update.cuh", "novelty.cuh", "cma.cuh")]
+    "rank.cuh", "update.cuh", "novelty.cuh", "cma.cuh", "map_elites.cuh")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-fmad=false",           # numerical contract: FMAs only where written (DESIGN.md section 4)
               "-Xcompiler", "-fPIC", "-shared"]
@@ -28,6 +28,10 @@ class ses_config(C.Structure):
 
 class ses_cma_params(C.Structure):
     _fields_ = [(n, C.c_double) for n in ("one_m_cs", "k_sigma", "one_m_cc", "k_c", "cc2", "c_keep", "c1", "cmu", "damp", "chi")]
+
+
+class ses_map_spec(C.Structure):
+    _fields_ = [("n_dims", C.c_int32), ("dims", C.c_int32 * 4), ("low", C.c_double * 4), ("width", C.c_double * 4), ("cells", C.c_int32 * 4)]
 
 
 # every symbol include/ses_b200.h declares: name -> (restype, argtypes)
@@ -64,6 +68,8 @@ SYMBOLS = {
     "ses_blend_shaped": (C.c_int, [_vp, _vp, _vp, _i32, _f64, _vp, _vp]),
     "ses_cma_sample": (C.c_int, [_vp, _u32, _vp, _vp, _vp, _vp, _vp]),
     "ses_cma_update": (C.c_int, [_vp, _u32, _vp, _vp, _i32, C.POINTER(ses_cma_params), _f64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "ses_map_insert": (C.c_int, [_vp, _u32, _f32, _vp, _vp, _vp, _vp, C.POINTER(ses_map_spec), _vp, _vp, _vp, _vp, _vp]),
+    "ses_map_select": (C.c_int, [_vp, _u32, C.POINTER(ses_map_spec), _vp, _vp, _vp, _vp, _vp, _vp]),
 }
 # include/ses_b200_test.h: only in the test build
 TEST_SYMBOLS = {

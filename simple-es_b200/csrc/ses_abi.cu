@@ -15,6 +15,7 @@
 #include <cstring>
 
 #include "cma.cuh"
+#include "map_elites.cuh"
 #include "novelty.cuh"
 #include "rank.cuh"
 #include "rollout_cartpole_mlp.cuh"
@@ -113,6 +114,10 @@ struct ses_handle {
     int k1_split = 1;
     int k1_sparse = 1;
     int *eval_counter = nullptr;   // work counter of ses_evaluate / ses_record launches (allocated by the first call)
+    // map_elites scratch (allocated by the first ses_map_* call, grown with the cell count): per-cell claims (all zero between
+    // calls: k_map_commit resets every claim it reads), the occupied-cell list, and the cell each rank entered
+    int *map_claim = nullptr, *map_list = nullptr, *map_enter = nullptr;
+    int map_cells = 0;
 
     int64_t launches = 0;
 };
@@ -246,6 +251,7 @@ extern "C" int ses_destroy(ses_handle *h)
     cudaFree(h->h_fitness); cudaFree(h->h_shaped); cudaFree(h->h_steps); cudaFree(h->h_order); cudaFree(h->h_total);
     cudaFree(h->e_parents); cudaFree(h->e_out); cudaFree(h->e_fitness); cudaFree(h->e_steps); cudaFree(h->e_order); cudaFree(h->e_total);
     cudaFree(h->eval_counter);
+    cudaFree(h->map_claim); cudaFree(h->map_list); cudaFree(h->map_enter);
     delete h;
     return 0;
 }
@@ -995,6 +1001,100 @@ extern "C" int ses_cma_update(ses_handle *h, uint32_t generation, const int32_t 
                                            parent_dev);
     h->launches += 1;
     CU(cudaGetLastError());
+    return 0;
+}
+
+// ------------------------------------------------------------------------------------------------
+// map_elites (DESIGN.md section 4.12)
+// ------------------------------------------------------------------------------------------------
+// The layout and the descriptor spec; *out := the spec as the kernels take it, *n_cells_out := the cell count
+static int map_check(const ses_handle *h, const ses_map_spec *spec, const char *fn, MapSpec *out, int *n_cells_out)
+{
+    if (h->cfg.group != 1 || h->cfg.n_head != 0 || h->cfg.antithetic)
+        return fail("%s: needs the map_elites layout (group = 1, n_head = 0, no antithetic pairs); this handle has group %d, n_head %d, "
+                    "antithetic %d", fn, h->cfg.group, h->cfg.n_head, h->cfg.antithetic);
+    if (spec->n_dims < 1 || spec->n_dims > MAP_MAX_DIMS) return fail("%s: n_dims must be in [1, %d] (got %d)", fn, MAP_MAX_DIMS, spec->n_dims);
+    long long n = 1;
+    for (int j = 0; j < spec->n_dims; ++j) {
+        if (spec->dims[j] < 0 || spec->dims[j] >= h->state_dim)
+            return fail("%s: dims[%d] = %d outside the final state [0, %d)", fn, j, spec->dims[j], h->state_dim);
+        for (int k = 0; k < j; ++k)
+            if (spec->dims[k] == spec->dims[j]) return fail("%s: dims[%d] = dims[%d] = %d: the dimensions must be distinct", fn, k, j, spec->dims[j]);
+        if (!std::isfinite(spec->low[j]) || !std::isfinite(spec->width[j]) || !(spec->width[j] > 0.0))
+            return fail("%s: dimension %d needs a finite low and a finite width > 0 (got low %g, width %g)", fn, j, spec->low[j], spec->width[j]);
+        if (spec->cells[j] < 1) return fail("%s: cells[%d] must be >= 1 (got %d)", fn, j, spec->cells[j]);
+        n *= spec->cells[j];
+        if (n > (1ll << 20)) return fail("%s: more than 2^20 cells (%lld after dimension %d)", fn, n, j);
+    }
+    if (n * h->D * 4 > (1ll << 32))
+        return fail("%s: %lld cells x %d parameters x 4 bytes = %lld bytes of elite weights exceed 4 GiB", fn, n, h->D, n * h->D * 4);
+    out->n_dims = spec->n_dims;
+    for (int j = 0; j < MAP_MAX_DIMS; ++j) {
+        const bool used = j < spec->n_dims;
+        out->dims[j] = used ? spec->dims[j] : 0;
+        out->low[j] = used ? spec->low[j] : 0.0;
+        out->width[j] = used ? spec->width[j] : 1.0;
+        out->cells[j] = used ? spec->cells[j] : 1;
+    }
+    *n_cells_out = (int)n;
+    return 0;
+}
+
+static int map_scratch(ses_handle *h, int n_cells, cudaStream_t st)
+{
+    if (!h->map_enter) CU(cudaMalloc(&h->map_enter, sizeof(int) * (size_t)h->cfg.population));
+    if (n_cells > h->map_cells) {
+        CU(cudaStreamSynchronize(st));          // the old scratch may still be read by earlier launches on this stream
+        cudaFree(h->map_claim); cudaFree(h->map_list);
+        h->map_claim = h->map_list = nullptr;
+        h->map_cells = 0;
+        CU(cudaMalloc(&h->map_claim, sizeof(int) * (size_t)n_cells));
+        CU(cudaMalloc(&h->map_list, sizeof(int) * (size_t)n_cells));
+        CU(cudaMemset(h->map_claim, 0, sizeof(int) * (size_t)n_cells));
+        h->map_cells = n_cells;
+    }
+    return 0;
+}
+
+extern "C" int ses_map_insert(ses_handle *h, uint32_t generation, float sigma, const float *parents_dev, const int32_t *order_dev,
+                              const double *fitness_dev, const double *bc_dev, const ses_map_spec *spec, double *F_dev, double *B_dev,
+                              int32_t *born_dev, float *W_dev, void *stream)
+{
+    if (!h) return fail("ses_map_insert: null handle");
+    if (!parents_dev || !order_dev || !fitness_dev || !bc_dev || !spec || !F_dev || !B_dev || !born_dev || !W_dev)
+        return fail("ses_map_insert: null argument");
+    MapSpec ms;
+    int n_cells = 0;
+    if (map_check(h, spec, "ses_map_insert", &ms, &n_cells)) return -1;
+    CU(cudaSetDevice(h->cfg.device));
+    cudaStream_t st = S(stream);
+    if (map_scratch(h, n_cells, st)) return -1;
+    const int P = h->cfg.population, grid = (P + 255) / 256;
+    k_map_claim<<<grid, 256, 0, st>>>(order_dev, fitness_dev, bc_dev, P, h->state_dim, ms, h->map_claim);
+    k_map_commit<<<grid, 256, 0, st>>>(order_dev, fitness_dev, bc_dev, P, h->state_dim, ms, h->map_claim, generation, F_dev, B_dev,
+                                       born_dev, h->map_enter);
+    const Layout lay{h->cfg.group, h->cfg.n_head, h->cfg.antithetic};
+    k_map_weights<<<P, 128, 0, st>>>(parents_dev, order_dev, h->map_enter, h->D, h->NQ, sigma, h->cfg.seed, generation, lay, W_dev);
+    CU(cudaGetLastError());
+    h->launches += 3;
+    return 0;
+}
+
+extern "C" int ses_map_select(ses_handle *h, uint32_t generation, const ses_map_spec *spec, const double *F_dev, const float *W_dev,
+                              const float *seed_row_dev, double *stats_dev, float *parents_dev, void *stream)
+{
+    if (!h) return fail("ses_map_select: null handle");
+    if (!spec || !F_dev || !W_dev || !seed_row_dev || !stats_dev || !parents_dev) return fail("ses_map_select: null argument");
+    MapSpec ms;
+    int n_cells = 0;
+    if (map_check(h, spec, "ses_map_select", &ms, &n_cells)) return -1;
+    CU(cudaSetDevice(h->cfg.device));
+    cudaStream_t st = S(stream);
+    if (map_scratch(h, n_cells, st)) return -1;
+    k_map_compact<<<1, MAP_COMPACT_THREADS, 0, st>>>(F_dev, n_cells, h->map_list, stats_dev);
+    k_map_gather<<<h->cfg.population, 256, 0, st>>>(W_dev, h->map_list, stats_dev, seed_row_dev, h->D, h->cfg.seed, generation, parents_dev);
+    CU(cudaGetLastError());
+    h->launches += 2;
     return 0;
 }
 

@@ -40,6 +40,8 @@ def population_layout(strategy, offspring_num, elite_num=None):
         return n, n, 1, 1                    # [mu, n-1 perturbed]
     if strategy == "sep_cma_es":
         return n, n, 0, 1                    # every offspring sampled (DESIGN.md section 4.11)
+    if strategy == "map_elites":
+        return n, 1, 0, n                    # offspring i = parent row i + sigma * noise (DESIGN.md section 4.12)
     if strategy == "simple_genetic":
         k = int(elite_num)
         g = n // k
@@ -102,6 +104,14 @@ def owned_ids(P, rank, world, block):
 def cma_params(k):
     """The ses_cma_params struct of sep_cma_constants(...) k."""
     return C.byref(_lib.ses_cma_params(**{f: float(k[f]) for f, _ in _lib.ses_cma_params._fields_}))
+
+
+def map_spec(dims, low, high, cells):
+    """The ses_map_spec struct of a map_elites descriptor: width = high - low in float64, once, on the host."""
+    n = len(dims)
+    return _lib.ses_map_spec(n_dims=n, dims=(C.c_int32 * 4)(*dims), low=(C.c_double * 4)(*[float(x) for x in low]),
+                             width=(C.c_double * 4)(*[float(h) - float(lo) for lo, h in zip(low, high)]),
+                             cells=(C.c_int32 * 4)(*cells))
 
 
 def _ptr(t):
@@ -297,6 +307,39 @@ class RolloutEngine:
         self._check(self.lib.ses_cma_update(self._h, int(generation), _ptr(order), _ptr(weights), int(consts["mu"]), cma_params(consts),
                                             sep_cma_threshold(consts, generation), _ptr(s), _ptr(mean), _ptr(c), _ptr(p_sigma),
                                             _ptr(p_c), _ptr(sigma), _ptr(parent), self._stream()))
+
+    # ------------------------------------------------------------------------------ map_elites
+    def _map_archive(self, spec, F, W, B=None, born=None):
+        n = 1
+        for j in range(spec.n_dims):
+            n *= int(spec.cells[j])
+        self._chk(F, torch.float64, n, "F")
+        self._chk(W, torch.float32, n * self.D, "W")
+        self._chk(B, torch.float64, n * self.state_dim, "B")
+        self._chk(born, torch.int32, 2 * n, "born")
+
+    def map_insert(self, generation, sigma, parents, order, fitness, bc, spec, F, B, born, W):
+        """Insert generation `generation` into the archive (DESIGN.md section 4.12), in place: F [n_cells] f64 (NaN = empty),
+        B [n_cells, state_dim] f64, born [n_cells, 2] i32 and W [n_cells, D] f32.  parents [P, D] f32 is the table the
+        generation was rolled out with, order [P] i32 rank_desc of fitness [P] f64, bc [P, state_dim] f64 the behaviours;
+        spec: map_spec(...)."""
+        self._chk(parents, torch.float32, self.P * self.D, "parents")
+        self._chk(order, torch.int32, self.P, "order")
+        self._chk(fitness, torch.float64, self.P, "fitness")
+        self._chk(bc, torch.float64, self.P * self.state_dim, "bc")
+        self._map_archive(spec, F, W, B, born)
+        self._check(self.lib.ses_map_insert(self._h, int(generation), float(sigma), _ptr(parents), _ptr(order), _ptr(fitness), _ptr(bc),
+                                            C.byref(spec), _ptr(F), _ptr(B), _ptr(born), _ptr(W), self._stream()))
+
+    def map_select(self, generation, spec, F, W, seed_row, stats, parents):
+        """The parent table of generation `generation` from the archive (F, W): parents [P, D] f32; stats [4] f64 := (occupied
+        cells, best cell or -1, its fitness, QD score).  seed_row [D] f32 fills every row while the archive is empty."""
+        self._map_archive(spec, F, W)
+        self._chk(seed_row, torch.float32, self.D, "seed_row")
+        self._chk(stats, torch.float64, 4, "stats")
+        self._chk(parents, torch.float32, self.P * self.D, "parents")
+        self._check(self.lib.ses_map_select(self._h, int(generation), C.byref(spec), _ptr(F), _ptr(W), _ptr(seed_row), _ptr(stats),
+                                            _ptr(parents), self._stream()))
 
     # ------------------------------------------------------------------------------ K1
     def rollout(self, generation, sigma, parents, fitness=None, steps=None, w_override=None, init_states=None,

@@ -6,6 +6,9 @@ generation print line (loop.py:89-91), wandb keys (loop.py:94-99), and
 ``logs/<env.name>/<%Y%m%d%H%M%S>/saved_models/ep_<n>.pt`` holding the elite's
 GymEnvModel-compatible state_dict every ``save_model_period`` generations (loop.py:40-47,101-104).
 
+map_elites only: rank 0 also saves the archive as ``archive_ep_<n>.pt`` next to ``ep_<n>.pt`` and prints one more line per
+generation (cells filled, best elite, QD score); wandb gets ``archive_coverage``, ``archive_best`` and ``archive_qd_score``.
+
 Opt-in (``engine.eval_every: N``): after every generation ep_num with ep_num % N == 0 the policy the loop saves
 (``elite_flat()``) is evaluated on ``engine.eval_episodes`` episodes (default 100, test.py's count) keyed by ep_num, so a
 resumed run reports what the uninterrupted one does; rank 0 prints one more line, wandb gets ``eval_mean_reward`` /
@@ -21,7 +24,7 @@ import torch
 
 from . import checkpoint
 from . import dist as sdist
-from .strategies import STRATEGIES
+from .strategies import STRATEGIES, MapElites
 
 
 class BaseESLoop(metaclass=ABCMeta):
@@ -97,6 +100,22 @@ class B200Loop(BaseESLoop):
         n = self.net_cfg
         return checkpoint.flat_to_state_dict(self.strategy.elite_flat(), int(n["num_state"]), int(n["num_action"]), bool(n["gru"]))
 
+    def archive_file(self):
+        """map_elites: the archive as saved in archive_ep_<n>.pt -- the occupied cells in ascending index with their grid
+        coordinates, fitness, behaviour, weights (flat, in checkpoint.state_dict_to_flat order) and birth, plus the
+        descriptor spec and the env / network sections that eval_es.py --archive needs."""
+        s = self.strategy
+        a = s.archive()
+        coords, rest = [], a["cells"].clone()
+        for n in reversed(s.cells):
+            coords.append(rest % n)
+            rest = rest // n
+        return {"cells": a["cells"], "coords": torch.stack(coords[::-1], dim=1), "fitness": a["fitness"], "behavior": a["behavior"],
+                "weights": a["weights"], "born_generation": a["born"][:, 0].clone(), "born_id": a["born"][:, 1].clone(),
+                "spec": {"behavior_dims": list(s.dims), "behavior_low": list(s.low), "behavior_high": list(s.high),
+                         "behavior_cells": list(s.cells)},
+                "env": dict(self.config["env"]), "network": dict(self.net_cfg), "generation": s.generation}
+
     def evaluate_elite(self, ep_num):
         """Returns of the policy elite_flat() on eval_episodes episodes keyed by ep_num: one eval_history entry."""
         start = time.time()
@@ -133,6 +152,12 @@ class B200Loop(BaseESLoop):
                 self.ep5_rewards.append(best_reward)
                 self._wandb.log({"ep5_mean_reward": sum(self.ep5_rewards) / len(self.ep5_rewards),
                                  "curr_sigma": curr_sigma})
+            if isinstance(s, MapElites):                     # 4 doubles the kernels wrote before the sync above
+                n_occ, n_cells, a_best, qd = s.archive_stats()
+                if self.rank == 0 and not self.quiet:
+                    print(f"  archive: {n_occ} / {n_cells} cells, best {a_best:.2f}, qd score {qd:.2f}")
+                if self._wandb is not None:
+                    self._wandb.log({"archive_coverage": n_occ / n_cells, "archive_best": a_best, "archive_qd_score": qd})
             if self.eval_every and ep_num % self.eval_every == 0:
                 _, n, mean, std, lo, hi, mlen, secs = self.evaluate_elite(ep_num)
                 if self.rank == 0 and not self.quiet:
@@ -142,6 +167,8 @@ class B200Loop(BaseESLoop):
                     self._wandb.log({"eval_mean_reward": mean, "eval_std_reward": std})
             if self.rank == 0 and self.save_model_period and self.save_model_period > 0 and ep_num % self.save_model_period == 0:
                 torch.save(self.elite_state_dict(), self.save_dir + "/saved_models" + f"/ep_{ep_num}.pt")
+                if isinstance(s, MapElites):
+                    torch.save(self.archive_file(), self.save_dir + "/saved_models" + f"/archive_ep_{ep_num}.pt")
                 if self.engine_cfg.get("save_state"):
                     torch.save(dict(s.state(), ep5_rewards=list(self.ep5_rewards)), self.save_dir + "/saved_models" + f"/resume_ep_{ep_num}.pt")
         return self.history

@@ -1,5 +1,5 @@
-"""Device-resident strategy state for the offspring strategies: the reference's three, and two opt-in additions: nsr_es
-(novelty search with reward) and sep_cma_es (separable CMA-ES).
+"""Device-resident strategy state for the offspring strategies: the reference's three, and three opt-in additions: nsr_es
+(novelty search with reward), sep_cma_es (separable CMA-ES) and map_elites (MAP-Elites).
 
 Each class keeps what the reference strategy keeps (learning_strategies/evolution/offspring_strategies.py)
 -- mu / elite table, sigma, Adam moments -- as a few small CUDA tensors, and never materialises the
@@ -7,10 +7,12 @@ population: offspring i of generation g is (parent(i), sigma, Philox(seed, g, i)
 generation: K1 rollout of this rank's slice, fitness exchange, K2 rank, K3 update -- the GPU form of
 ``results = p.map(RolloutWorker, ...); strategy.evaluate(results)`` (loop.py:66-84).
 """
+import math
+
 import torch
 
 from . import dist as sdist
-from .engine import RolloutEngine, cyclic_block, owned_ids, population_layout, sep_cma_constants, shard_bounds
+from .engine import ENV_SPECS, RolloutEngine, cyclic_block, map_spec, owned_ids, population_layout, sep_cma_constants, shard_bounds
 
 
 class _Base:
@@ -112,6 +114,27 @@ class _Base:
                 sdist.exchange_fitness_masked(self.fitness, self._not_mine)
             else:
                 sdist.exchange_fitness(self.fitness, self.lo, self.hi)
+
+    def _final_state_output(self):
+        """Have K1 store every episode's final state (nsr_es, map_elites): final_states [P, E, state_dim] and the behaviours
+        bc [P, state_dim] that _behaviors() computes from them."""
+        e, dev = self.engine, self.engine.device
+        self.final_states = torch.zeros((self.P, e.E, e.state_dim), dtype=torch.float64, device=dev)
+        e.set_final_states(self.final_states)
+        self.bc = torch.empty((self.P, e.state_dim), dtype=torch.float64, device=dev)
+        if self.shard and not hasattr(self, "_not_mine"):
+            mask = torch.ones(self.P, dtype=torch.bool)
+            mask[torch.from_numpy(owned_ids(self.P, *self.shard))] = False
+            self._not_mine = mask.to(dev)
+
+    def _behaviors(self):
+        """After K1: every rank's final states on every rank, exactly, then bc := their means over episodes."""
+        if sdist.world()[1] > 1:                       # every rank gets every row, exactly; then all compute the same
+            if self.shard:
+                sdist.exchange_fitness_masked(self.final_states, self._not_mine)
+            else:
+                sdist.exchange_fitness(self.final_states, self.lo, self.hi)
+        self.engine.behavior(self.final_states, out=self.bc)
 
     def _rollout_and_rank(self, shaped=False):
         self._rollout_and_exchange()
@@ -280,19 +303,13 @@ class NoveltyES(OpenAIES):
         super().__init__(strategy_cfg, *a, **kw)
         e, dev = self.engine, self.engine.device
         self._run_key.update(novelty_k=self.novelty_k, novelty_weight=self.novelty_weight)
-        self.final_states = torch.zeros((self.P, e.E, e.state_dim), dtype=torch.float64, device=dev)
-        e.set_final_states(self.final_states)
-        self.bc = torch.empty((self.P, e.state_dim), dtype=torch.float64, device=dev)
+        self._final_state_output()
         self.novelty = torch.empty(self.P, dtype=torch.float64, device=dev)
         self.novelty_order = torch.empty(self.P, dtype=torch.int32, device=dev)
         self.shaped_f = torch.empty(self.P, dtype=torch.float64, device=dev)
         self.shaped_n = torch.empty(self.P, dtype=torch.float64, device=dev)
         self.archive = torch.empty((16, e.state_dim), dtype=torch.float64, device=dev)   # grows by doubling
         self.n_archive = 0
-        if self.shard and not hasattr(self, "_not_mine"):
-            mask = torch.ones(self.P, dtype=torch.bool)
-            mask[torch.from_numpy(owned_ids(self.P, *self.shard))] = False
-            self._not_mine = mask.to(dev)
 
     def _reserve(self, n):
         if n > self.archive.shape[0]:
@@ -304,12 +321,7 @@ class NoveltyES(OpenAIES):
     def step(self):
         e = self.engine
         self._rollout_and_exchange()                   # K1 also stores every episode's final state (set_final_states)
-        if sdist.world()[1] > 1:                       # every rank gets every row, exactly; then all compute the same
-            if self.shard:
-                sdist.exchange_fitness_masked(self.final_states, self._not_mine)
-            else:
-                sdist.exchange_fitness(self.final_states, self.lo, self.hi)
-        e.behavior(self.final_states, out=self.bc)
+        self._behaviors()
         self._reserve(self.n_archive + 1)
         self.archive[self.n_archive].copy_(self.bc[0])   # mu's behaviour joins the archive before novelty is measured
         self.n_archive += 1
@@ -426,4 +438,158 @@ class SepCMAES(_Base):
             getattr(self, k).copy_(st[k])
 
 
-STRATEGIES = {c.name: c for c in (OpenAIES, SimpleEvolution, SimpleGenetic, NoveltyES, SepCMAES)}
+MAP_MAX_CELLS = 1 << 20
+MAP_MAX_WEIGHT_BYTES = 1 << 32
+
+
+def _map_state_dim(env_cfg, engine_cfg):
+    name = env_cfg["name"]
+    if name not in ENV_SPECS:
+        raise ValueError("env %r is not supported by the B200 engine" % (name,))
+    sd = ENV_SPECS[name][2]
+    return 4 * int(engine_cfg.get("n_agents", 2)) if sd is None else sd
+
+
+def _map_params(cfg, state_dim, D):
+    """(offspring_num, dims, low, high, cells) of a map_elites strategy section, validated against the final-state size
+    state_dim and the parameter count D (DESIGN.md section 4.12)."""
+    allowed = {"name", "init_sigma", "sigma_decay", "offspring_num", "behavior_dims", "behavior_low", "behavior_high", "behavior_cells"}
+    unknown = sorted(set(cfg) - allowed)
+    if unknown:
+        raise ValueError("strategy map_elites: unknown key(s) %s (allowed: %s)" % (", ".join(unknown), ", ".join(sorted(allowed))))
+    missing = sorted(k for k in allowed - {"name"} if k not in cfg)
+    if missing:
+        raise ValueError("strategy map_elites: missing key(s) %s" % ", ".join(missing))
+
+    def num(x):
+        return not isinstance(x, bool) and isinstance(x, (int, float))
+
+    def intg(x):
+        return not isinstance(x, bool) and isinstance(x, int)
+    n = cfg["offspring_num"]
+    if not intg(n) or n < 2:
+        raise ValueError("strategy map_elites: offspring_num must be an integer >= 2 (got %r)" % (n,))
+    for k in ("init_sigma", "sigma_decay"):
+        if not num(cfg[k]) or not math.isfinite(cfg[k]):
+            raise ValueError("strategy map_elites: %s must be a finite number (got %r)" % (k, cfg[k]))
+    dims, low, high, cells = (cfg[k] for k in ("behavior_dims", "behavior_low", "behavior_high", "behavior_cells"))
+    for k, v in (("behavior_dims", dims), ("behavior_low", low), ("behavior_high", high), ("behavior_cells", cells)):
+        if not isinstance(v, (list, tuple)) or not 1 <= len(v) <= 4:
+            raise ValueError("strategy map_elites: %s must be a list of 1 to 4 entries (got %r)" % (k, v))
+    if not len(dims) == len(low) == len(high) == len(cells):
+        raise ValueError("strategy map_elites: behavior_dims, behavior_low, behavior_high and behavior_cells must have one entry per "
+                         "descriptor dimension (got %d, %d, %d, %d)" % (len(dims), len(low), len(high), len(cells)))
+    if not all(intg(d) and 0 <= d < state_dim for d in dims):
+        raise ValueError("strategy map_elites: behavior_dims must be indices into the final state [0, %d) (got %r)" % (state_dim, dims))
+    if len(set(dims)) != len(dims):
+        raise ValueError("strategy map_elites: behavior_dims must be distinct (got %r)" % (dims,))
+    for j, (lo, hi) in enumerate(zip(low, high)):
+        if not (num(lo) and num(hi) and math.isfinite(lo) and math.isfinite(hi)):
+            raise ValueError("strategy map_elites: behavior_low / behavior_high must be finite numbers (dimension %d: %r, %r)" % (j, lo, hi))
+        if not float(hi) - float(lo) > 0.0:
+            raise ValueError("strategy map_elites: behavior_low must be below behavior_high (dimension %d: %r, %r)" % (j, lo, hi))
+    if not all(intg(c) and c >= 1 for c in cells):
+        raise ValueError("strategy map_elites: behavior_cells must be integers >= 1 (got %r)" % (cells,))
+    n_cells = math.prod(cells)
+    if n_cells > MAP_MAX_CELLS:
+        raise ValueError("strategy map_elites: %s = %d cells exceed 2^20 = %d" % (" x ".join(map(str, cells)), n_cells, MAP_MAX_CELLS))
+    if n_cells * D * 4 > MAP_MAX_WEIGHT_BYTES:
+        raise ValueError("strategy map_elites: %d cells x %d parameters x 4 bytes = %d bytes of elite weights exceed 4 GiB = %d"
+                         % (n_cells, D, n_cells * D * 4, MAP_MAX_WEIGHT_BYTES))
+    return int(n), [int(d) for d in dims], [float(x) for x in low], [float(x) for x in high], [int(c) for c in cells]
+
+
+class MapElites(_Base):
+    """MAP-Elites (Mouret & Clune 2015; opt-in, the reference has no such strategy): an archive of one elite per cell of a grid
+    over final-state coordinates.  Every generation, parent row i is the elite of an occupied cell drawn by Philox, offspring i
+    is that row + sigma * noise, and the best-ranked offspring of each cell replaces the cell's elite if its fitness is higher.
+    The archive (fitness F, behaviour B, birth and weights W of every cell) lives on the device (DESIGN.md section 4.12)."""
+    name = "map_elites"
+
+    def __init__(self, strategy_cfg, env_cfg, network_cfg, eval_ep_num, seed, device, engine_cfg):
+        from .checkpoint import param_shapes
+        D = sum(math.prod(shape) for _, shape in param_shapes(int(network_cfg["num_state"]), int(network_cfg["num_action"]),
+                                                             bool(network_cfg["gru"])))
+        _, self.dims, self.low, self.high, self.cells = _map_params(strategy_cfg, _map_state_dim(env_cfg, engine_cfg), D)
+        if engine_cfg.get("antithetic", False):
+            raise ValueError("map_elites does not support engine.antithetic: with one parent row per offspring there are no pairs to mirror")
+        super().__init__(strategy_cfg, env_cfg, network_cfg, eval_ep_num, seed, device, engine_cfg)
+        e, dev = self.engine, self.engine.device
+        self._run_key.update(behavior_dims=list(self.dims), behavior_low=list(self.low), behavior_high=list(self.high),
+                             behavior_cells=list(self.cells))
+        self._final_state_output()
+        self.spec = map_spec(self.dims, self.low, self.high, self.cells)
+        self.n_cells = math.prod(self.cells)
+        self.F = torch.full((self.n_cells,), float("nan"), dtype=torch.float64, device=dev)
+        self.B = torch.full((self.n_cells, e.state_dim), float("nan"), dtype=torch.float64, device=dev)
+        self.born = torch.full((self.n_cells, 2), -1, dtype=torch.int32, device=dev)
+        self.W = torch.zeros((self.n_cells, self.D), dtype=torch.float32, device=dev)
+        self.seed_row = torch.zeros(self.D, dtype=torch.float32, device=dev)     # network.zero_init(), or engine.init_from
+        self.stats = torch.zeros(4, dtype=torch.float64, device=dev)
+        self._select()
+
+    def _select(self):
+        self.engine.map_select(self.generation, self.spec, self.F, self.W, self.seed_row, self.stats, self.parents)
+
+    def step(self):
+        e = self.engine
+        self._rollout_and_exchange()                   # K1 also stores every episode's final state (set_final_states)
+        self._behaviors()
+        e.rank_desc(self.fitness, order=self.order)
+        e.map_insert(self.generation, self.sigma, self.parents, self.order, self.fitness, self.bc, self.spec, self.F, self.B, self.born, self.W)
+        self.sigma *= self.decay
+        self.curr_sigma = self.sigma
+        self.generation += 1
+        self._select()                                 # the parent table of the next generation, and the archive's statistics
+        self._mark(2)
+
+    def archive_stats(self):
+        """(occupied cells, n_cells, best fitness, QD score) after the last insertion; reads 4 doubles from the device."""
+        n_occ, _, best, qd = self.stats.tolist()
+        return int(n_occ), self.n_cells, best, qd
+
+    def elite_flat(self):
+        c = int(self.stats[1].item())
+        return self.W[c] if c >= 0 else self.seed_row
+
+    def load_elite(self, flat):
+        """Start from a saved policy: the seed row S := flat (every parent row while the archive is empty)."""
+        flat = torch.as_tensor(flat, dtype=torch.float32).reshape(-1)
+        if flat.numel() != self.D:
+            raise ValueError("checkpoint has %d parameters, the configured network has %d" % (flat.numel(), self.D))
+        self.seed_row.copy_(flat.to(self.seed_row.device))
+        self._select()
+
+    def archive(self):
+        """The occupied cells as CPU tensors: cells [n] i64 ascending, fitness [n] f64, behavior [n, state_dim] f64,
+        weights [n, D] f32, born [n, 2] i64 (generation, offspring id)."""
+        cells = torch.nonzero(~torch.isnan(self.F)).reshape(-1)
+        return {"cells": cells.cpu(), "fitness": self.F[cells].cpu(), "behavior": self.B[cells].cpu(), "weights": self.W[cells].cpu(),
+                "born": self.born[cells].to(torch.int64).cpu()}
+
+    def state(self):
+        st = super().state()
+        st["archive"] = self.archive()
+        st["seed_row"] = self.seed_row.detach().cpu().clone()
+        return st
+
+    def load_state(self, st):
+        super().load_state(st)
+        a = st["archive"]
+        n = a["cells"].numel()
+        if a["weights"].shape != (n, self.D) or a["behavior"].shape != (n, self.B.shape[1]) or n and int(a["cells"].max()) >= self.n_cells:
+            raise ValueError("resume state's archive does not fit this run (%d cells of %d parameters)" % (self.n_cells, self.D))
+        cells = a["cells"].to(self.F.device)
+        self.F.fill_(float("nan"))
+        self.B.fill_(float("nan"))
+        self.born.fill_(-1)
+        self.W.zero_()
+        self.F[cells] = a["fitness"].to(self.F.device)
+        self.B[cells] = a["behavior"].to(self.B.device)
+        self.born[cells] = a["born"].to(self.born.device, torch.int32)
+        self.W[cells] = a["weights"].to(self.W.device)
+        self.seed_row.copy_(st["seed_row"])
+        self._select()
+
+
+STRATEGIES = {c.name: c for c in (OpenAIES, SimpleEvolution, SimpleGenetic, NoveltyES, SepCMAES, MapElites)}
